@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (one process per GPU under torchrun for N>1)
     python bench.py --impl reference --gpus N --steps K --warmup W   # CPU arm: the reference's own Python on the host cores
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR  # + what the last timed step returned, as DIR/*.npy
 
 Workload (BASELINE.json configs[1]): HoverAviary single-drone PPO-rollout shape, 65,536 parallel envs per GPU,
 Physics.DYN, ActionType.RPM, KIN observation (72 floats), FP32, 240 Hz sim / 30 Hz ctrl (8 substeps per step),
@@ -65,7 +66,13 @@ def parse():
     ap.add_argument("--no-others", action="store_true", help="skip other_configs (BASELINE configs[2..4])")
     ap.add_argument("--ref-kind", default="auto", choices=["auto", "python", "port"],
                     help="reference arm: the staged reference Python (oracle/_ref) or the C oracle port")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (obs, reward, terminated, truncated of the env set it stepped; "
+                         "rank 0) as DIR/<name>.npy, so that two builds can be compared output for output")
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
+    return a
 
 
 def workload_name(a):
@@ -307,6 +314,25 @@ def graph_of(torch, fn):
     return g
 
 
+DUMP_MAX_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, outputs):
+    """Writes `outputs` (name -> array with the env axis first) as DIR/<name>.npy in float64 (float64 arrays) or float32 (the
+    rest).  Beyond DUMP_MAX_BYTES in all, every array keeps the same fixed, seeded sample of envs, listed in env_index.npy."""
+    arrs = {k: np.ascontiguousarray(v, dtype=np.float64 if v.dtype == np.float64 else np.float32) for k, v in outputs.items()}
+    E = len(next(iter(arrs.values())))
+    per_env = sum(v.nbytes for v in arrs.values()) / E
+    if per_env * E > DUMP_MAX_BYTES:
+        n = int((DUMP_MAX_BYTES - 4096) // (per_env + 8))          # 4 KB for the .npy headers, 8 B per env for env_index
+        idx = np.sort(np.random.default_rng(0).choice(E, n, replace=False))
+        arrs = {k: v[idx] for k, v in arrs.items()}
+        arrs["env_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrs.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
 def measure_config(torch, timer, make_env, make_action, nsets, steps, trials=3):
     """µs per step of one BASELINE shape: `nsets` rotating env sets, `steps` steps in one CUDA graph, best of `trials` windows,
     max over ranks."""
@@ -444,10 +470,12 @@ def b200_arm(a):
     pool = [torch.cuda.Stream(device=dev) for _ in range(nstreams - 1)]
 
     def run_steps(n, nstreams=nstreams, pool=pool, k0=0):
+        """Steps k0 .. k0+n-1; returns what the last step returned (views of the buffers it writes, also under capture)."""
+        out = None
         if nstreams == 1:
             for k in range(k0, k0 + n):
-                envs[k % nsets]._sim.step(acts[k % period])
-            return
+                out = envs[k % nsets]._sim.step(acts[k % period])
+            return out
         # fork: every pool stream waits for the caller's stream; set j always runs on stream j % nstreams (its own steps stay
         # ordered); join: the caller's stream waits for every pool stream.  All of it is capturable.
         main = torch.cuda.current_stream()
@@ -458,11 +486,12 @@ def b200_arm(a):
         for k in range(k0, k0 + n):
             j = (k % nsets) % nstreams
             with torch.cuda.stream(main if j == 0 else pool[j - 1]):
-                envs[k % nsets]._sim.step(acts[k % period])
+                out = envs[k % nsets]._sim.step(acts[k % period])
         for st in pool:
             ev = torch.cuda.Event()
             ev.record(st)
             main.wait_event(ev)
+        return out
 
     # warm-up (also touches every buffer); whole cycles so that the observation ping-pong phase is back where it started
     wu = max(3, a.warmup)
@@ -490,6 +519,10 @@ def b200_arm(a):
     reps, tail = divmod(K, gper) if mode == "cycles" else (0, 0)
     graphs = None
     graph_error = None
+    last = {}           # timed unit -> what its last step returned
+
+    def unit_steps(key, n, k0=0):
+        last[key] = run_steps(n, k0=k0)
     if mode != "direct":
         try:
             if mode == "single":
@@ -499,12 +532,12 @@ def b200_arm(a):
 
                 def unit(i):
                     gev[i][0].record()
-                    run_steps(K, k0=i * K)
+                    unit_steps(i, K, k0=i * K)
                     gev[i][1].record()
                 graphs = [graph_of(torch, (lambda i=i: unit(i))) for i in range(m)]
             else:
-                graphs = {"main": graph_of(torch, lambda: run_steps(gper)),
-                          "tail": graph_of(torch, lambda: run_steps(tail)) if tail else None,
+                graphs = {"main": graph_of(torch, lambda: unit_steps("main", gper)),
+                          "tail": graph_of(torch, lambda: unit_steps("tail", tail)) if tail else None,
                           "comp": graph_of(torch, lambda: run_steps(gper - tail, k0=tail)) if tail else None}
         except Exception as ex:          # never lose the measurement to a capture problem: fall back to direct launches
             graphs = None
@@ -515,7 +548,7 @@ def b200_arm(a):
 
     def timed_unit():
         if mode == "direct":
-            run_steps(K, k0=nxt[0] * K)
+            unit_steps("direct", K, k0=nxt[0] * K)
             nxt[0] = (nxt[0] + 1) % m
         elif mode == "single":
             graphs[nxt[0]].replay()
@@ -534,13 +567,21 @@ def b200_arm(a):
         while nxt[0] != 0:
             timed_unit()
 
-    # bring the clocks to their loaded state (untimed): ~0.3 s of the same work
-    t_end = time.perf_counter() + 0.3
-    n_pre = 0
-    while time.perf_counter() < t_end or n_pre < 2:
+    def last_key():     # the unit whose last step was the last timed step
+        if mode == "single":
+            return (nxt[0] - 1) % m
+        return "direct" if mode == "direct" else ("tail" if tail else "main")
+
+    # bring the clocks to their loaded state (untimed): the same work for ~0.3 s on a B200 (34,880 steps at 65,536 envs,
+    # launch-bound below).  Counted in steps, not timed, so that every run steps the env sets through the same sequence
+    # and the outputs of the timed steps do not depend on the speed of the build.  Auto-resets come in bursts, so where
+    # the timed windows fall in an episode moves the figure by ~1 %: the count is what 0.3 s of timed pre-warm reached
+    # on a B200 (1000 W limit) with 20-step windows, 1,744 of them (profiles/bench_prewarm.txt).  A faster build
+    # pre-warms for proportionally less time.
+    pre_steps = 34_880 * 65_536 // max(E, 65_536)
+    for n_pre in range(1, max(2, -(-pre_steps // K)) + 1):
         timed_unit()
         after_unit()
-        n_pre += 1
         if n_pre % 8 == 0:
             torch.cuda.synchronize()
     torch.cuda.synchronize()
@@ -549,8 +590,11 @@ def b200_arm(a):
     windows, per_rank_all = [], []
     # long enough for the host to enqueue the whole window behind it (direct mode: ~10 us of host time per launch)
     sleep_cycles = 400_000 + (40_000 * K if mode == "direct" else 60 * min(K, 4096))
-    for _ in range(trials):
+    dumped = None
+    for i in range(trials):
         ms_local = timer.window(timed_unit, sleep_cycles, events=gev[nxt[0]] if mode == "single" else None)
+        if a.dump_outputs and rank == 0 and i == trials - 1:     # before any later step overwrites the buffers
+            dumped = dict(zip(("obs", "reward", "terminated", "truncated"), (t.cpu().numpy() for t in last[last_key()])))
         after_unit()
         ms_max, per = timer.max_over_ranks(ms_local)
         windows.append(ms_max)
@@ -745,6 +789,8 @@ def b200_arm(a):
             "episode_stats": {"episodes": stats[0], "mean_return": stats[1] / max(stats[0], 1),
                               "mean_length": stats[2] / max(stats[0], 1), "env_steps": stats[6], "how": stats_how},
         }
+        if dumped is not None:
+            dump_outputs(a.dump_outputs, dumped)
         print(json.dumps(line), flush=True)
     for e in envs:
         e.close()
@@ -753,6 +799,7 @@ def b200_arm(a):
 
 
 def main():
+    sys.dont_write_bytecode = True      # the project's modules are imported below: the bench writes nothing into the tree
     a = parse()
     if a.impl == "reference":
         reference_arm(a)

@@ -445,13 +445,15 @@ def test_cuda_bulk_copy_path_matches_the_per_thread_path(act, flags, precision, 
 
 
 def test_oracle_matches_the_staged_reference_on_this_box():
-    """The CPU arm of bench.py runs the unmodified reference Python staged under oracle/_ref.  On the GPU box (where
-    /root/reference does not exist) replay random configurations in that copy and in the oracle: the checker of every parity
-    test here is pinned to the live reference on this very machine, not only to the committed fixtures."""
+    """The CPU arm of bench.py runs the unmodified upstream Python staged under oracle/_ref.  Where that copy exists, replay
+    random configurations in it and in the oracle on the GPU machine itself: the checker of every parity test here is then
+    pinned to the live upstream code, not only to the committed fixtures.  The upstream sources are not part of this
+    repository (__graft_entry__.build() stages them from GPD_REFERENCE)."""
     import json
     ref = os.path.join(ROOT, "oracle", "_ref")
     if not os.path.isdir(os.path.join(ref, "gym_pybullet_drones")):
-        pytest.skip("oracle/_ref not staged (python oracle/stage_reference.py in the build container)")
+        pytest.skip("needs the upstream gym-pybullet-drones sources, which this repository does not contain: build() "
+                    "stages them into oracle/_ref when GPD_REFERENCE points at a checkout of them")
     out = subprocess.run([sys.executable, os.path.join(ROOT, "oracle", "fuzz_vs_reference.py"), "--ref", ref, "--seeds", "24"],
                          capture_output=True, text=True, timeout=600, cwd=ROOT)
     lines = [l for l in out.stdout.splitlines() if l.startswith("{")]
