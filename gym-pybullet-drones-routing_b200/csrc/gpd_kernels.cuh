@@ -364,11 +364,15 @@ __device__ __forceinline__ void step_substep(const StepArgs<R>& a, State<R>& s, 
             // The gate |roll|,|pitch| < pi/2 of the rpy snapshot (BaseAviary.py:346-347,518,742) needs only the signs of
             // the atan2/asin arguments: |atan2(y,x)| < pi/2 <=> x > 0 (or x = y = 0); Bullet's gimbal branch
             // (|s| >= 0.99999) returns pitch = +-pi/2 and fails the gate, otherwise |asin(s)| < pi/2.  Exact in both
-            // precisions up to atan2 results that ROUND to pi/2 (|y/x| > 1e16): three libm calls per substep saved.
+            // precisions except where atan2 ROUNDS to pi/2: for x > 0 the correctly rounded double atan2(y, x) = pi/2 - x/|y|
+            // equals double(pi/2) once x/|y| <= (pi/2 - double(pi/2)) + 2^-53 = 1.7225e-16 (roll = +-pi/2 exactly, x a
+            // rounding residue), and the reference's gate is then false; FP64 tests that bound.  Three libm calls per
+            // substep saved.
             const R sarg = R(-2) * (s.qx * s.qz - s.qw * s.qy);
             const R rx = s.qw * s.qw - s.qx * s.qx - s.qy * s.qy + s.qz * s.qz, ry = R(2) * (s.qy * s.qz + s.qw * s.qx);
             const bool gimbal = sarg <= R(-0.99999) || sarg >= R(0.99999);
-            const R roll = gimbal ? R(0) : ((rx > R(0) || (rx == R(0) && ry == R(0))) ? R(0) : R(GPD_PI));
+            const bool upright = M<R>::is_double ? (rx > R(0) && M<R>::abs(ry) * R(1.7225464241988331e-16) < rx) : rx > R(0);
+            const R roll = gimbal ? R(0) : ((upright || (rx == R(0) && ry == R(0))) ? R(0) : R(GPD_PI));
             const R pitch = gimbal ? R(GPD_PI) : R(0);
             if (ground_effect(P, rpm_r, s.pz, m, roll, pitch, gnd)) pg = gnd;
         }
