@@ -215,6 +215,17 @@ static inline void unchain(gpd_sim* s, void* stream = nullptr, bool all = false)
     else g_chain.set(s->cfg.device, (cudaStream_t)stream, false, 0);
 }
 
+// Chained-state handles (SimPtrs): writes the state of every tile in chained state back into sP / sV / sWz / ep_ret, reading
+// position and velocity from the latest observation, and marks those tiles as held in the arrays.  Every entry point that
+// reads or writes the state other than the bulk step calls it first, on its own stream.  A step launched behind it must not
+// be chained (it would not wait for it): callers on the step path unchain the stream.
+static int sync_state(gpd_sim* s, void* stream)
+{
+    if (!s->a32.state_in_obs) return GPD_OK;
+    CU(launch_state_sync(s->a32, (const float*)s->last_obs, s->lc.grid, (cudaStream_t)stream));
+    return GPD_OK;
+}
+
 static int action_width(int act)
 {
     switch (act) {
@@ -413,6 +424,16 @@ static int build_args(gpd_sim* s, StepArgs<R>& a)
         const bool rpm_act = c.action_type == GPD_ACT_RPM || c.action_type == GPD_ACT_ONE_D_RPM;
         ev = getenv("GPD_AUX_ALWAYS");
         a.skip_aux = (sizeof(R) == 4 && rpm_act && c.physics_flags == 0 && c.env_kind != GPD_ENV_CTRL && !(ev && atoi(ev))) ? 1 : 0;
+        // of those, single-drone sims on the bulk kernel chain position and velocity through the observation (SimPtrs): 48 B
+        // per env-step less state traffic
+        ev = getenv("GPD_STATE_IN_OBS");
+        a.state_in_obs = (a.skip_aux && c.num_drones == 1 && s->bulk_ok && s->bulk_direct == 2 && !(ev && atoi(ev) == 0)) ? 1 : 0;
+    }
+    if (a.state_in_obs) {
+        V* sr;
+        if ((rc = dev_alloc(s, &sr, (size_t)s->D))) return rc;
+        a.sR = sr;
+        s->lc_bulk.smem += 16;      // row 0's old kin[0..3] in front of the tile (BulkSmem)
     }
     a.tma_edge_bytes = s->tma_edge_bytes;
     a.bulk_direct = s->bulk_direct;
@@ -709,6 +730,8 @@ int gpd_reset(gpd_sim* s, const uint8_t* env_mask, const void* obs_prev, void* o
     if (obs_out && obs_out == obs_prev) return fail(GPD_ERR_INVALID, "obs_prev must not alias obs_out");
     CU(use_device(s->cfg.device));
     unchain(s, stream);
+    int rc = sync_state(s, stream);
+    if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     if (s->cfg.precision == GPD_F64) {
         StepArgs<double> a = s->a64;
@@ -721,6 +744,20 @@ int gpd_reset(gpd_sim* s, const uint8_t* env_mask, const void* obs_prev, void* o
     }
     if (obs_out) { s->last_obs = obs_out; ++s->obs_seq; }
     return GPD_OK;
+}
+
+// the bulk copies need 16-byte aligned actions / observations (see step_impl)
+static bool bulk_step(const gpd_sim* s, const void* actions, const void* obs_prev, const void* obs_out)
+{
+    return s->bulk_ok && (((uintptr_t)actions | (uintptr_t)obs_prev | (uintptr_t)obs_out) & 15) == 0;
+}
+
+// Chained-state handles: the bulk step takes position and velocity of a chained tile from obs_prev, which must then be the
+// observation this handle wrote last (or was given through gpd_note_latest_obs).  Any other step, or one on the per-thread
+// kernel, must first move the state back into the arrays (sync_state), on a stream the whole step is ordered behind.
+static bool step_needs_sync(const gpd_sim* s, const void* actions, const void* obs_prev, const void* obs_out)
+{
+    return s->a32.state_in_obs && (!bulk_step(s, actions, obs_prev, obs_out) || obs_prev != s->last_obs);
 }
 
 static int step_impl(gpd_sim* s, const void* actions, const void* obs_prev, void* obs_out, void* reward, uint8_t* terminated,
@@ -743,9 +780,14 @@ static int step_impl(gpd_sim* s, const void* actions, const void* obs_prev, void
     // the per-thread kernel.  Reward / flag arrays that are not (rows of a [T][E] uint8 trajectory buffer) only switch those
     // three outputs to plain stores: a sim keeps ONE kernel, so its FP32 results do not depend on the caller's buffer layout
     // (the two kernels agree bit for bit in FP64; in FP32 only up to the compiler's FMA contraction choices).
-    const uintptr_t al = (uintptr_t)actions | (uintptr_t)obs_prev | (uintptr_t)obs_out;
     const uintptr_t al_out = (uintptr_t)reward | (uintptr_t)terminated | (uintptr_t)truncated;
-    const bool bulk = s->bulk_ok && (al & 15) == 0;
+    const bool bulk = bulk_step(s, actions, obs_prev, obs_out);
+    // a step issued in chunks on several streams (ncta > 0) is synced by its caller, before the fork to the chunk streams
+    if (ncta == 0 && step_needs_sync(s, actions, obs_prev, obs_out)) {
+        int rc = sync_state(s, stream);
+        if (rc) return rc;
+        unchain(s, stream);
+    }
     const int out_plain = ((al_out & 15) != 0 || host_io) ? 1 : 0;     // outputs in mapped host memory: plain stores by the threads
     LaunchCfg lc = bulk ? s->lc_bulk : s->lc;
     if (ncta > 0) lc.grid = ncta;       // a sub-range of the CTAs (chunked host-mirror step); cta0 shifts the block index
@@ -1107,6 +1149,11 @@ int gpd_step_mirror_begin(gpd_sim* s, const void* actions, const void* d_obs_pre
         CU(mirror_rows_d2h(s, m.row + s->A, m.d_kin_t, 12, st));
     } else {
         // fork: every chunk stream starts behind what the caller's stream holds so far (a window rebuild, earlier steps)
+        if (step_needs_sync(s, s->h_act, d_obs_prev, d_obs_out)) {      // ahead of the fork: every chunk stream waits for it
+            int rc = sync_state(s, stream);
+            if (rc) return rc;
+            unchain(s, stream);
+        }
         CU(cudaEventRecord(m.ev_fork, st));
         const int64_t G = s->lc.grid;
         const size_t act_row = (size_t)s->A * 4;        // RL envs: float32 actions
@@ -1210,6 +1257,8 @@ int gpd_get_state(gpd_sim* s, void* state20, void* rpy_rates, void* pid_state, i
     if (!s) return fail(GPD_ERR_INVALID, "null handle");
     CU(use_device(s->cfg.device));
     unchain(s, stream);
+    int rc = sync_state(s, stream);
+    if (rc) return rc;
     if (s->cfg.precision == GPD_F64)
         CU(launch_get_state<double>(s->a64, (const float*)s->last_obs, (double*)state20, (double*)rpy_rates, (double*)pid_state, step_counter, (cudaStream_t)stream));
     else
@@ -1231,6 +1280,8 @@ int gpd_set_state(gpd_sim* s, const void* state20, const void* rpy_rates, const 
     if (!s) return fail(GPD_ERR_INVALID, "null handle");
     CU(use_device(s->cfg.device));
     unchain(s, stream);
+    int rc = sync_state(s, stream);
+    if (rc) return rc;
     if (s->cfg.precision == GPD_F64)
         CU(launch_set_state<double>(s->a64, (const double*)state20, (const double*)rpy_rates, (const double*)pid_state, step_counter, (cudaStream_t)stream));
     else
@@ -1334,6 +1385,8 @@ int gpd_count_nonfinite(gpd_sim* s, long long* out_host, void* stream)
     if (!s || !out_host) return fail(GPD_ERR_INVALID, "gpd_count_nonfinite: null argument");
     CU(use_device(s->cfg.device));
     unchain(s, stream);
+    int rc = sync_state(s, stream);
+    if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     unsigned long long* cnt = (unsigned long long*)s->stats_out;       // reuse the 64-byte scratch
     CU(cudaMemsetAsync(cnt, 0, sizeof(unsigned long long), st));
@@ -1458,6 +1511,8 @@ int gpd_adjacency(gpd_sim* s, double neighbourhood_radius, void* out, void* stre
     if (!s || !out) return fail(GPD_ERR_INVALID, "gpd_adjacency: null argument");
     CU(use_device(s->cfg.device));
     unchain(s, stream);
+    int rc = sync_state(s, stream);
+    if (rc) return rc;
     if (s->cfg.precision == GPD_F64) CU(launch_adjacency<double>(s->a64, neighbourhood_radius, (double*)out, (cudaStream_t)stream));
     else CU(launch_adjacency<float>(s->a32, (float)neighbourhood_radius, (float*)out, (cudaStream_t)stream));
     return GPD_OK;

@@ -80,6 +80,34 @@ cudaError_t launch_transpose_cols(const float* obs, int64_t D, int W, int j0, in
     return cudaGetLastError();
 }
 
+// ============================================================================================
+// Chained-state handles (SimPtrs, StepArgs::state_in_obs): the state of every tile in chained state back into the arrays
+// (position / velocity from the latest observation row, rates / episode return from sR), then the tile's flag cleared.
+// One CTA per bulk tile.
+// ============================================================================================
+__global__ void __launch_bounds__(128) state_sync_kernel(const StepArgs<float> a, const float* __restrict__ obs)
+{
+    unsigned long long* flag = a.tile_seq + (int64_t)blockIdx.x * 4 + 1;
+    if (*flag == 0ull || !obs) return;
+    const int64_t d = (int64_t)blockIdx.x * a.DPB + threadIdx.x;
+    if ((int)threadIdx.x < a.DPB && d < a.D) {
+        const float* k = obs + d * a.W;
+        const float4 r = a.sR[d];
+        a.p.sP[d] = make_float4(k[0], k[1], k[2], r.x);
+        a.p.sV[d] = make_float4(k[6], k[7], k[8], r.y);
+        a.p.sWz[d] = r.z;
+        if (a.p.ep_ret) a.p.ep_ret[d] = r.w;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) *flag = 0ull;
+}
+
+cudaError_t launch_state_sync(const StepArgs<float>& a, const float* obs_latest, int64_t tiles, cudaStream_t st)
+{
+    state_sync_kernel<<<(unsigned)tiles, (a.DPB + 31) / 32 * 32, 0, st>>>(a, obs_latest);
+    return cudaGetLastError();
+}
+
 // job-wide statistics from the all-gathered per-rank vectors {episodes, ret, len, ret^2, min, max, env_steps, terminated}:
 // sums in rank order (deterministic), min/max over the ranks that finished at least one episode
 __global__ void stats_combine_kernel(const double* __restrict__ g, int nranks, double* __restrict__ out8)

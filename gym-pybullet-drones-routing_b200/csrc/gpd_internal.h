@@ -59,6 +59,10 @@ struct DevPid {
 //   Lean FP32 KIN sims (StepArgs::skip_aux) do not write them per step: both are bit-exact functions of the observation
 //   row (kin[9..11]; newest ring slot + counter) and are re-derived on demand; *aux_auth says which copy is authoritative.
 //   pid[k*D + d], k = 0..8
+//   Chained-state handles (StepArgs::state_in_obs): the bulk step keeps position and velocity only in the kin part of the
+//   latest observation row (kin[0..2], kin[6..8]: the float32 state itself), rates and episode return in StepArgs::sR =
+//   (rates.xyz, ep_ret); a tile whose flag (tile_seq[4 * tile + 1]) is set holds its state so, and launch_state_sync writes
+//   it back into sP / sV / sWz / ep_ret for every other reader or writer of the state.
 template <typename R>
 struct SimPtrs {
     typename Vec4<R>::type* sP;
@@ -114,10 +118,13 @@ struct StepArgs {
     int32_t tpc;            // bulk path, per call: tiles per CTA (0/1 = one; chained launches may take GPD_BULK_MAX_TPC)
     int32_t tile_end;       // bulk path, per call: first tile not covered by this launch
     int32_t bulk_direct;    // bulk path: what bypasses shared memory (0 nothing, 1 the small per-env arrays, 2 the state vectors too)
+    int32_t state_in_obs;   // lean FP32 single-drone sims on the bulk kernel: position / velocity chained through the observation (SimPtrs)
     SimPtrs<R> p;
     DevDrone<R> drone;
     DevPid<R> pid;
     double pyb_freq, episode_len;
+    // after everything the other kernels read, so that their parameter layout does not depend on it
+    typename Vec4<R>::type* sR;   // [D] chained-state handles only: (rates.x, rates.y, rates.z, ep_ret)
 };
 
 struct LaunchCfg {
@@ -152,6 +159,7 @@ template <typename R> cudaError_t launch_drag(const DevDrone<R>& d, int64_t n, c
 template <typename R> cudaError_t launch_downwash(const DevDrone<R>& d, int64_t E, int N, const R* pos, R* out,
                                                   cudaStream_t st);
 template <typename R> cudaError_t launch_adjacency(const StepArgs<R>& a, R radius, R* out, cudaStream_t st);
+cudaError_t launch_state_sync(const StepArgs<float>& a, const float* obs_latest, int64_t tiles, cudaStream_t st);
 template <typename R> cudaError_t launch_nonfinite(const StepArgs<R>& a, unsigned long long* out, cudaStream_t st);
 template <typename R> cudaError_t launch_rollout_pid(const StepArgs<R>& a, int n_steps, const R* waypoints, int n_wp,
                                                      int32_t* wp_counters, R* action, cudaStream_t st);

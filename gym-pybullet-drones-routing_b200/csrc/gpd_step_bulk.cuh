@@ -9,7 +9,10 @@
 // gpd_kernels.cuh) and issues, on ONE mbarrier,
 //     the observation tile   T rows x W floats, CONTIGUOUS in global memory, read from obs_prev at +A floats: in shared
 //                            memory row r then holds [old kin[4..11] | old ring slots 1..B-1 | 16 stray bytes], i.e. the
-//                            shifted ring already sits where the new row wants it (BaseRLAviary.py:187,317-318)
+//                            shifted ring already sits where the new row wants it (BaseRLAviary.py:187,317-318).  The
+//                            chained-state variant (bulk_chain_variant) reads whole rows into shared memory 16 bytes in
+//                            front of the tile instead: the same layout, the stray bytes being row r+1's old kin[0..3], so
+//                            every row's whole old kin is in shared memory
 //     (bulk_direct < 2)      the state tiles sP, sQ, sV (16/32 B per env); (bulk_direct == 0) sWz, step counter, episode
 //                            return and the action tile too — by default (bulk_direct = 2) every thread fetches those itself
 //                            and only the observation tile occupies shared memory (BulkSmem)
@@ -67,7 +70,8 @@ __device__ __forceinline__ void slide_row(float4* r, int W4, const float* act)
     r[W4 - 1] = funnel4<A>(lo, make_float4(act[0], act[1], act[2], 0.f));
 }
 
-// shared-memory carve-up of one tile (every region starts 16-byte aligned because T % 16 == 0).  `direct` (StepArgs::
+// shared-memory carve-up of one tile (every region starts 16-byte aligned because T % 16 == 0): `front` bytes (16 in the
+// chained-state variant: row 0's old kin[0..3] when A == 4; 0 otherwise), then the observation tile.  `direct` (StepArgs::
 // bulk_direct) says what does NOT go through shared memory — shared memory per env is what bounds the number of tiles
 // in flight per SM, and with it the launch's throughput (tiles in flight / lifetime of a tile):
 //     0  everything staged: 370 B per env (FP32, W = 72)                            9 tiles of 64 envs per SM
@@ -77,9 +81,9 @@ __device__ __forceinline__ void slide_row(float4* r, int W4, const float* act)
 template <typename R>
 struct BulkSmem {
     unsigned char* base;
-    int T, W, direct;
-    __device__ float* obs() const { return reinterpret_cast<float*>(base); }
-    __device__ V4<R>* sP() const { return reinterpret_cast<V4<R>*>(base + (size_t)T * W * 4); }
+    int T, W, direct, front;
+    __device__ float* obs() const { return reinterpret_cast<float*>(base + front); }
+    __device__ V4<R>* sP() const { return reinterpret_cast<V4<R>*>(base + front + (size_t)T * W * 4); }
     __device__ V4<R>* sQ() const { return sP() + T; }
     __device__ V4<R>* sV() const { return sQ() + T; }
     __device__ unsigned char* after_state() const { return reinterpret_cast<unsigned char*>(sP() + (direct >= 2 ? 0 : 3 * T)); }
@@ -107,8 +111,14 @@ struct BulkPre {
     R wz;
     int32_t cnt;
     float ep;
-    V4<R> p4, q4, v4;       // direct == 2
+    V4<R> p4, q4, v4;       // direct == 2 (a tile in chained state: rates.x / rates.y from sR, xyz from the old kin in shared memory)
 };
+
+// The one kernel variant that takes StepArgs::state_in_obs (lean FP32 single-drone sims, direct == 2): it reads position and
+// velocity of a tile in chained state from the old kin in shared memory and rates / episode return from sR (36 B of state per
+// env-step each way instead of 60), writes sQ, sR and the counter only, and leaves the tile in chained state.
+template <typename R, int KIND, bool MULTI>
+__host__ __device__ constexpr bool bulk_chain_variant() { return KIND == GPD_K_LEAN && !MULTI && !M<R>::is_double; }
 
 // One thread's share of a tile: state / action / counters from shared memory, the arithmetic of gpd::step_kernel, results
 // back into the tile (plus the few per-drone extras that live only in global memory).  `sub` = timeline slot or -1.
@@ -117,6 +127,7 @@ __device__ __forceinline__ void bulk_tile_physics(const StepArgs<R>& a, const Bu
                                                   int64_t row0, int rows, int tl)
 {
     constexpr bool LEAN = KIND == GPD_K_LEAN, HAS_PID = KIND == GPD_K_PID;
+    const bool chained = bulk_chain_variant<R, KIND, MULTI>() && a.state_in_obs;
     const DevDrone<R>& P = a.drone;
     const int64_t d = row0 + t;             // drone; tiles hold whole envs (T and row0 are multiples of N)
     const int le = MULTI ? t / a.N : t;     // env within the tile
@@ -309,7 +320,10 @@ __device__ __forceinline__ void bulk_tile_physics(const StepArgs<R>& a, const Bu
 
     // ---- everything back into the tile ----
     if (active) {
-        if (direct >= 2) {
+        if (chained) {                      // position and velocity travel in the observation row written below
+            a.p.sQ[d] = M<R>::make4(s.qx, s.qy, s.qz, s.qw);
+            a.sR[d] = M<R>::make4(s.wx, s.wy, s.wz, (R)ep_new);
+        } else if (direct >= 2) {
             a.p.sP[d] = M<R>::make4(s.px, s.py, s.pz, s.wx);
             a.p.sQ[d] = M<R>::make4(s.qx, s.qy, s.qz, s.qw);
             a.p.sV[d] = M<R>::make4(s.vx, s.vy, s.vz, s.wy);
@@ -320,10 +334,10 @@ __device__ __forceinline__ void bulk_tile_physics(const StepArgs<R>& a, const Bu
         }
         const int32_t cnt_new = done ? 0 : cnt + a.S;                   // BaseAviary.py:382
         if (direct) {
-            a.p.sWz[d] = s.wz;
+            if (!chained) a.p.sWz[d] = s.wz;
             if (lead) {
                 a.p.counter[e] = cnt_new;
-                if (a.auto_reset) a.p.ep_ret[e] = ep_new;
+                if (a.auto_reset && !chained) a.p.ep_ret[e] = ep_new;
             }
         } else {
             sm.sWz()[t] = s.wz;
@@ -400,7 +414,8 @@ step_kernel_bulk(const __grid_constant__ StepArgs<R> a)
     const int t = threadIdx.x;
     const int T = a.DPB;
     const int direct = a.bulk_direct;
-    BulkSmem<R> sm{ smem_raw, T, a.W, direct };
+    constexpr bool CHAIN = bulk_chain_variant<R, KIND, MULTI>();
+    BulkSmem<R> sm{ smem_raw, T, a.W, direct, CHAIN ? 16 : 0 };
     // Tiles of this CTA: one by default.  A chained launch (gpd_set_step_chaining) gives every CTA up to `tpc` tiles, strided by
     // the grid so that at any moment the CTAs cover a contiguous range: the tiles run one after the other through the SAME
     // shared-memory buffer, all claims are issued up front in one round trip, and a tile is published while the NEXT tile's
@@ -459,14 +474,15 @@ step_kernel_bulk(const __grid_constant__ StepArgs<R> a)
         if (t == 0) {
             fence_proxy_async_global();         // generic-proxy writes of the tile's previous step (ragged tails) -> bulk reads
             const uint32_t v4b = (uint32_t)sizeof(V4<R>);
-            // A == 4: read at +A floats (already shifted); the last tile of the buffer must not read past its end: its final row
-            // loses the 16 stray bytes.  A < 4: whole rows, unshifted (slide_row)
-            const uint32_t shift = a.A == 4 ? 4u : 0u;
+            // A == 4: already shifted, i.e. read at +A floats (the last tile of the buffer must not read past its end: its final
+            // row loses the 16 stray bytes) or, in the chained-state variant, whole rows landing 16 bytes in front of the tile.
+            // A < 4: whole rows, unshifted (slide_row)
+            const uint32_t shift = a.A == 4 && !CHAIN ? 4u : 0u;
             const uint32_t ob = a.obs_prev ? (uint32_t)rows * a.W * 4 - ((shift && row0 + rows >= a.D) ? 16u : 0u) : 0u;
             const uint32_t st = (uint32_t)rows * v4b, sc = (uint32_t)T * (uint32_t)sizeof(R), i4 = (uint32_t)T * 4u;
             const uint32_t total = ob + (direct >= 2 ? 0u : 3 * st) + (direct ? 0u : (uint32_t)rows * 16u + sc + i4 + (a.auto_reset ? i4 : 0u));
             mbar_expect_tx(&bar, total);
-            if (ob) bulk_g2s(sm.obs(), a.obs_prev + row0 * a.W + shift, ob, &bar);
+            if (ob) bulk_g2s(CHAIN && a.A == 4 ? sm.obs() - 4 : sm.obs(), a.obs_prev + row0 * a.W + shift, ob, &bar);
             if (direct < 2) {
                 bulk_g2s(sm.sP(), a.p.sP + row0, st, &bar);
                 bulk_g2s(sm.sQ(), a.p.sQ + row0, st, &bar);
@@ -482,6 +498,10 @@ step_kernel_bulk(const __grid_constant__ StepArgs<R> a)
         BulkPre<R> pre;
         pre.act = make_float4(0.f, 0.f, 0.f, 0.f); pre.wz = R(0); pre.cnt = 0; pre.ep = 0.f;
         pre.p4 = pre.q4 = pre.v4 = M<R>::make4(R(0), R(0), R(0), R(0));
+        // this tile's state lives in the observation chain (set by its previous step, cleared by launch_state_sync; the
+        // claim above acquired it together with the tile).  A step without obs_prev is preceded by a sync on the host.
+        const bool from_obs = CHAIN && a.state_in_obs && a.obs_prev &&
+                              a.tile_seq[(int64_t)bid * 4 + 1] != 0ull;
         if (direct && t < rows) {               // the thread's own small inputs: in flight under the bulk loads
             const int64_t d = row0 + t;
             if (a.A == 4) {
@@ -492,11 +512,17 @@ step_kernel_bulk(const __grid_constant__ StepArgs<R> a)
                 if (a.A > 1) pre.act.y = __ldg(ap + 1);
                 if (a.A > 2) pre.act.z = __ldg(ap + 2);
             }
-            pre.wz = a.p.sWz[d];
+            if (!from_obs) pre.wz = a.p.sWz[d];
             const int64_t e = MULTI ? d / a.N : d;      // every drone of an env reads the env's counter / return (one address per env)
             pre.cnt = a.p.counter[e];
-            if (a.auto_reset) pre.ep = a.p.ep_ret[e];
-            if (direct >= 2) { pre.p4 = a.p.sP[d]; pre.q4 = a.p.sQ[d]; pre.v4 = a.p.sV[d]; }
+            if (from_obs) {
+                const V4<R> r4 = a.sR[d];
+                pre.q4 = a.p.sQ[d];
+                pre.p4.w = r4.x; pre.v4.w = r4.y; pre.wz = r4.z; pre.ep = (float)r4.w;
+            } else {
+                if (a.auto_reset) pre.ep = a.p.ep_ret[e];
+                if (direct >= 2) { pre.p4 = a.p.sP[d]; pre.q4 = a.p.sQ[d]; pre.v4 = a.p.sV[d]; }
+            }
         }
         if (!a.obs_prev && t < rows) {          // no previous observation: all-zero ring (BaseRLAviary.py:153-154)
             float* r = sm.obs() + (size_t)t * a.W;
@@ -510,6 +536,15 @@ step_kernel_bulk(const __grid_constant__ StepArgs<R> a)
         }
         mbar_wait(&bar, (uint32_t)(it & 1));
         if (a.timeline && t == 0) a.timeline[(int64_t)bid * 8 + 2] = gtime();
+        if (from_obs) {
+            if (t < rows) {                     // the old row starts 16 bytes in front of the new one when A == 4 (kin[0..3] at
+                                                // the end of row t-1's slot), at it otherwise
+                const float* k = sm.obs() + (size_t)t * a.W - (a.A == 4 ? 4 : 0);
+                pre.p4.x = k[0]; pre.p4.y = k[1]; pre.p4.z = k[2];
+                pre.v4.x = k[6]; pre.v4.y = k[7]; pre.v4.z = k[8];
+            }
+            if (a.A == 4) __syncthreads();      // row t-1's newest ring slot overwrites row t's old kin[0..3]
+        }
 
         bulk_tile_physics<R, KIND, MULTI>(a, sm, pre, t, row0, rows, bid);
         fence_proxy_async_smem();               // this thread's shared-memory writes -> the bulk stores below
@@ -537,6 +572,8 @@ step_kernel_bulk(const __grid_constant__ StepArgs<R> a)
             }
             asm volatile("cp.async.bulk.commit_group;" ::: "memory");
             bulk_tile_stats<R>(a, sm, bid, MULTI ? rows / a.N : rows);
+            // published with the tile: its next step reads position and velocity from this observation
+            if (CHAIN && a.state_in_obs && !from_obs) a.tile_seq[(int64_t)bid * 4 + 1] = 1ull;
         }
     }
 

@@ -145,6 +145,11 @@ int gpd_reset(gpd_sim* sim, const uint8_t* env_mask, const void* obs_prev, void*
  *   obs_prev  dev, the observation written by the previous gpd_step/gpd_reset on this handle: the RL observation
  *             carries the action ring (BaseRLAviary.py:317-318), so the shifted history is read from it.
  *             NULL = all-zero ring. Ignored for the Ctrl env. Must not alias obs_out.
+ *             FP32 single-drone KIN sims with an RPM-type action and no force model (GPD_STATE_IN_OBS=0 turns this off)
+ *             keep position and velocity ONLY in the kin part of the latest observation (kin[0..2], kin[6..8]: the
+ *             float32 state itself): the next step reads them from there, so an in-place edit of the returned observation
+ *             is an edit of the env's state. A step whose obs_prev is neither the handle's latest obs_out nor the buffer
+ *             given to gpd_note_latest_obs takes its state from the handle's own copy instead, like every other handle.
  *   obs_out   dev [E][N][W]: float32 (RL) / Real (Ctrl)
  *   reward    dev [E] Real (NULL allowed); terminated/truncated dev [E] uint8 (NULL allowed)
  *   terminal_kin dev [E][N][12] float32 or NULL: with auto_reset, the 12 kinematic observation entries of a
@@ -236,7 +241,8 @@ int gpd_reset_mirror(gpd_sim* sim, const uint8_t* env_mask, const void* d_obs_pr
  * passed as obs_out - the same buffer the next gpd_step needs intact as obs_prev. */
 int gpd_get_state(gpd_sim* sim, void* state20, void* rpy_rates, void* pid_state, int32_t* step_counter, void* stream);
 /* Tells the library which device buffer now holds the latest observation (a caller that copied it elsewhere and is about to
- * release the buffer it passed as obs_out). Only FP32 KIN sims with an RPM-type action and no force model read it back. */
+ * release the buffer it passed as obs_out). Only FP32 KIN sims with an RPM-type action and no force model read it back;
+ * for the single-drone ones it then carries the position and velocity the next step starts from (see gpd_step). */
 int gpd_note_latest_obs(gpd_sim* sim, const void* obs);
 int gpd_set_state(gpd_sim* sim, const void* state20, const void* rpy_rates, const void* pid_state,
                   const int32_t* step_counter, void* stream);
