@@ -645,6 +645,8 @@ int gpd_create(const gpd_config* cfg, gpd_sim** out)
         s->bulk_ok = eligible && (ev ? atoi(ev) != 0 : s->W * 4 <= 512);
         s->lc_bulk.threads = (DPB + 31) / 32 * 32; s->lc_bulk.grid = L.grid; s->lc_bulk.smem = bsm; s->lc_bulk.pdl = 0;   // whole warps
     }
+    int bps_dbg = 0;
+    double waves_dbg = 0;
     {   // programmatic dependent launch: measured to help only launches of at most ~2 CTAs per SM (the CTA launch and the
         // parameter fetch overlap the previous kernel's tail); with a full wave the early-resident CTAs all issue their
         // loads at the same instant after the wait and the burst costs more than the overlap gains
@@ -670,11 +672,14 @@ int gpd_create(const gpd_config* cfg, gpd_sim** out)
         const char* ev = getenv("GPD_PDL");
         s->lc.pdl = ev ? atoi(ev) : ((s->tile_dep || s->lc.grid <= 296) ? 1 : 0);
         s->lc_bulk.pdl = s->lc.pdl;
-        if (getenv("GPD_DEBUG_LAYOUT"))
-            fprintf(stderr, "[gpd] %d CTAs/SM, %.2f waves: tile_dep %d, pdl %d, bulk path %d\n", bps, waves, s->tile_dep, s->lc.pdl, (int)s->bulk_ok);
+        bps_dbg = bps; waves_dbg = waves;
     }
     if (s->lc.grid > 0x7fffffffLL) { delete s; return fail(GPD_ERR_INVALID, "too many envs for one launch"); }
     int rc = cfg->precision == GPD_F64 ? build_args(s, s->a64) : build_args(s, s->a32);
+    if (rc == GPD_OK && getenv("GPD_DEBUG_LAYOUT"))      // one line per handle: every create-time choice of the step's data path
+        fprintf(stderr, "[gpd] %d CTAs/SM, %.2f waves: tile_dep %d, pdl %d, bulk path %d, tile %d, tiles %lld, tma %d, tma_edge %d, "
+                "bulk_tpc %d, state_in_obs %d\n", bps_dbg, waves_dbg, s->tile_dep, s->lc.pdl, (int)s->bulk_ok, s->dpb,
+                (long long)s->lc.grid, (int)s->tma_ok, s->tma_edge, s->bulk_tpc, s->a32.state_in_obs);
     if (rc == GPD_OK) { cudaError_t e = cudaMalloc((void**)&s->stats_out, 8 * sizeof(double)); if (e != cudaSuccess) rc = fail(GPD_ERR_ALLOC, "cudaMalloc failed"); }
     if (rc != GPD_OK) { gpd_destroy(s); return rc; }
     // start in the reset state (BaseAviary.__init__ ends with _housekeeping + _updateAndStoreKinematicInformation)
@@ -771,7 +776,10 @@ static int step_impl(gpd_sim* s, const void* actions, const void* obs_prev, void
     cudaStream_t st = (cudaStream_t)stream;
     CUtensorMap tp, to, te;
     bool have = false;
-    if (s->tma_ok && obs_prev) {
+    // actions or observations that are not 16-byte aligned (step_into on offset views) take the per-thread kernel's scalar
+    // variant (launch_step), which has no TMA path for 4-wide actions
+    const bool al16 = (((uintptr_t)actions | (uintptr_t)obs_prev | (uintptr_t)obs_out) & 15) == 0;
+    if (s->tma_ok && obs_prev && al16) {
         have = get_tmap(s, obs_prev, false, &tp) && get_tmap(s, obs_out, false, &to);
         if (have && s->tma_edge) have = get_tmap(s, obs_prev, true, &te);
     }

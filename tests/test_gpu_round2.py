@@ -507,7 +507,7 @@ def test_cuda_chained_stepping_across_eager_and_captured_launches(precision):
 
 def test_cuda_default_tile_sizes():
     """gpd_create's measured layout defaults for the single-drone RL shapes (gpd_grid_size = number of tiles): 128-env tiles for
-    lean FP32 sims of 37,888..262,144 envs and for FP64 / force-model sims, 64-env tiles otherwise (profiles/r02/sweep_b14/b16)."""
+    lean FP32 sims of 37,888..262,144 envs (both ends included) and for FP64 / force-model sims, 64-env tiles otherwise (profiles/r02/sweep_b14/b16)."""
     L = _lib.load()
     def tiles(E, precision="f32", **over):
         sim = make_sim(_kw(**over), E, precision, auto_reset=True)
@@ -515,7 +515,7 @@ def test_cuda_default_tile_sizes():
         sim.close()
         return g
     assert tiles(65536) == 512 and tiles(262144) == 2048 and tiles(37888) == 296
-    assert tiles(16384) == 256 and tiles(37887) == 592 and tiles(600000) == 9375
+    assert tiles(16384) == 256 and tiles(37887) == 592 and tiles(600000) == 9375 and tiles(262145) == 4097
     assert tiles(65536, act="pid", freq=48, model=DroneModel.CF2P) == 1024        # 3-wide actions: 64-env tiles
     assert tiles(65536, "f64") == 512 and tiles(20000, "f64") == 157
     assert tiles(65536, flags=3) == 512                                            # force models: 128
