@@ -31,7 +31,7 @@ SYMBOLS = [
     "gpd_set_timeline_buffer", "gpd_count_nonfinite", "gpd_set_targets", "gpd_mirror_alloc", "gpd_mirror_free",
     "gpd_mirror_attach", "gpd_mirror_row", "gpd_step_mirror", "gpd_step_mirror_begin", "gpd_step_mirror_end",
     "gpd_reset_mirror", "gpd_nccl_unique_id", "gpd_nccl_comm_init", "gpd_nccl_comm_destroy", "gpd_adjacency",
-    "gpd_set_step_chaining",
+    "gpd_set_step_chaining", "gpd_rollout",
 ]
 
 
@@ -154,6 +154,7 @@ def load(path: str | None = None):
     L.gpd_force_drag.argtypes = [C.c_int, C.c_int, C.POINTER(DroneParamsC), i64, vp, vp, vp, vp, vp]
     L.gpd_force_downwash.argtypes = [C.c_int, C.c_int, C.POINTER(DroneParamsC), i64, i32, vp, vp, vp]
     L.gpd_rollout_pid.argtypes = [vp, i32, vp, i32, vp, vp, vp]
+    L.gpd_rollout.argtypes = [vp, i32, vp, vp, vp, vp, u8p, u8p, vp, vp, vp]
     L.gpd_episode_stats.argtypes = [vp, C.POINTER(dbl), C.c_int, vp, vp]
     L.gpd_set_targets.argtypes = [vp, C.POINTER(dbl), C.c_int]
     L.gpd_mirror_alloc.argtypes = [i64, i64, C.POINTER(vp)]

@@ -1388,6 +1388,45 @@ int gpd_rollout_pid(gpd_sim* s, int32_t n_ctrl_steps, const void* waypoints, int
     return GPD_OK;
 }
 
+int gpd_rollout(gpd_sim* s, int32_t n_steps, const void* actions, const void* obs_prev, void* obs_out,
+                void* reward, uint8_t* terminated, uint8_t* truncated, void* traj, void* terminal_kin, void* stream)
+{
+    if (!s) return fail(GPD_ERR_INVALID, "null handle");
+    if (n_steps < 1) return fail(GPD_ERR_INVALID, "gpd_rollout: n_steps must be >= 1");
+    if (!actions || !obs_out) return fail(GPD_ERR_INVALID, "gpd_rollout: actions and obs_out are required");
+    const bool ctrl = s->cfg.env_kind == GPD_ENV_CTRL;
+    if (ctrl) obs_prev = nullptr;
+    if (obs_out == obs_prev || obs_out == actions || (traj && (traj == obs_out || traj == actions)) ||
+        (terminal_kin && (terminal_kin == obs_out || terminal_kin == traj)))
+        return fail(GPD_ERR_INVALID, "gpd_rollout: aliased buffers");
+    if (((uintptr_t)actions | (uintptr_t)obs_prev | (uintptr_t)obs_out | (uintptr_t)traj | (uintptr_t)terminal_kin) & 15)
+        return fail(GPD_ERR_INVALID, "gpd_rollout: actions, observations, traj and terminal_kin must be 16-byte aligned");
+    CU(use_device(s->cfg.device));
+    cudaStream_t st = (cudaStream_t)stream;
+    unchain(s, stream);                 // the next step is not launched programmatically behind the rollout
+    int rc = sync_state(s, stream);     // chained-state tiles back into the arrays: the rollout reads and writes those
+    if (rc) return rc;
+    // the step kernel's tiles without its DMA warp: one statistics slot per CTA, as gpd_create allocated them
+    LaunchCfg lc{};
+    lc.threads = s->lc.threads - s->copy_threads;
+    lc.grid = s->lc.grid;
+    lc.smem = smem_bytes(s->cfg.precision == GPD_F64, false, s->cfg.num_drones > 1, s->dpb, s->dpb / s->cfg.num_drones);
+    if (s->cfg.precision == GPD_F64) {
+        StepArgs<double> a = s->a64;
+        a.actions = actions; a.obs_prev = (const float*)obs_prev; a.obs_out = obs_out; a.reward = (double*)reward;
+        a.terminated = terminated; a.truncated = truncated; a.terminal_kin = (float*)terminal_kin;
+        CU(launch_rollout<double>(a, n_steps, traj, lc, st));
+    } else {
+        StepArgs<float> a = s->a32;
+        a.actions = actions; a.obs_prev = (const float*)obs_prev; a.obs_out = obs_out; a.reward = (float*)reward;
+        a.terminated = terminated; a.truncated = truncated; a.terminal_kin = (float*)terminal_kin;
+        CU(launch_rollout<float>(a, n_steps, traj, lc, st));
+    }
+    s->last_obs = obs_out;
+    ++s->obs_seq;
+    return GPD_OK;
+}
+
 int gpd_count_nonfinite(gpd_sim* s, long long* out_host, void* stream)
 {
     if (!s || !out_host) return fail(GPD_ERR_INVALID, "gpd_count_nonfinite: null argument");

@@ -163,5 +163,7 @@ cudaError_t launch_state_sync(const StepArgs<float>& a, const float* obs_latest,
 template <typename R> cudaError_t launch_nonfinite(const StepArgs<R>& a, unsigned long long* out, cudaStream_t st);
 template <typename R> cudaError_t launch_rollout_pid(const StepArgs<R>& a, int n_steps, const R* waypoints, int n_wp,
                                                      int32_t* wp_counters, R* action, cudaStream_t st);
+// gpd_rollout: n_steps control steps of StepArgs::actions ([n_steps][D][A]) in one launch; traj as in include/gpd.h
+template <typename R> cudaError_t launch_rollout(const StepArgs<R>& a, int n_steps, void* traj, const LaunchCfg& lc, cudaStream_t st);
 
 }  // namespace gpd

@@ -305,13 +305,10 @@ __device__ __forceinline__ void init_state(const StepArgs<R>& a, int64_t d, int 
     s.wx = s.wy = s.wz = R(0);
 }
 
-// _preprocessAction for the PID-family action types (BaseRLAviary.py:193-235).
+// _preprocessAction for the PID-family action types (BaseRLAviary.py:193-235), on the DSLPID state st[9] held by the caller.
 template <typename R>
-__device__ __forceinline__ void pid_action(const StepArgs<R>& a, int64_t d, const State<R>& s, const float* act, R rpm[4])
+__device__ __forceinline__ void pid_action_st(const StepArgs<R>& a, const State<R>& s, const float* act, R (&st)[9], R rpm[4])
 {
-    R st[9];
-#pragma unroll
-    for (int k = 0; k < 9; ++k) st[k] = a.p.pid[(int64_t)k * a.D + d];
     R tp[3], trpy[3] = { R(0), R(0), R(0) }, tv[3] = { R(0), R(0), R(0) }, tr[3] = { R(0), R(0), R(0) }, pe[3], ye;
     if (a.action_type == GPD_ACT_PID) {
         // BaseAviary._calculateNextStep (BaseAviary.py:1105-1147), step_size = 1
@@ -337,6 +334,16 @@ __device__ __forceinline__ void pid_action(const StepArgs<R>& a, int64_t d, cons
         tp[0] = s.px + R(0.1) * R(0); tp[1] = s.py + R(0.1) * R(0); tp[2] = s.pz + R(0.1) * R(act[0]);
     }
     pid_compute(a.pid, a.ctrl_dt, s.px, s.py, s.pz, s.qx, s.qy, s.qz, s.qw, s.vx, s.vy, s.vz, tp, trpy, tv, tr, st, rpm, pe, ye);
+}
+
+// the same, with the DSLPID state of drone d read from and written back to a.p.pid
+template <typename R>
+__device__ __forceinline__ void pid_action(const StepArgs<R>& a, int64_t d, const State<R>& s, const float* act, R rpm[4])
+{
+    R st[9];
+#pragma unroll
+    for (int k = 0; k < 9; ++k) st[k] = a.p.pid[(int64_t)k * a.D + d];
+    pid_action_st(a, s, act, st, rpm);
 #pragma unroll
     for (int k = 0; k < 9; ++k) a.p.pid[(int64_t)k * a.D + d] = st[k];
 }

@@ -158,6 +158,21 @@ class BaseAviary:
         obs, rew, term, trunc = self._sim.step(action)
         return obs, rew, term.view(torch.bool), trunc.view(torch.bool), self._computeInfo()
 
+    def rollout(self, actions, return_traj: bool = False):
+        """K control steps of a given action schedule in one launch: the same as ``for k: step(actions[k])`` when the
+        intermediate observations are not read.  ``actions``: CUDA tensor (K, E, N, A).  Returns ``(obs, rewards,
+        terminated, truncated, info)``: the observation after the last step, rewards / flags of shape (K, E) (bool flags);
+        ``info["traj"]`` holds each step's kinematic part (K, E, N, 12) (the whole (K, E, N, 20) row for the Ctrl env)
+        when ``return_traj``."""
+        self._state_cache = None
+        self._numpy_io = False
+        out = self._sim.rollout(actions, traj=return_traj)
+        obs, rew, term, trunc = out[:4]
+        info = self._computeInfo()
+        if return_traj:
+            info = dict(info, traj=out[4])
+        return obs, rew, term.view(torch.bool), trunc.view(torch.bool), info
+
     def render(self, mode='human', close=False):
         """Text output of env 0 (BaseAviary.py:387-412)."""
         st = self._state()[0][0].cpu().numpy()

@@ -193,6 +193,53 @@ class BatchedSim:
         _lib.check(self.lib.gpd_step(self.h, _ptr(actions), _ptr(obs_prev), _ptr(obs_out), _ptr(reward), _ptr(terminated),
                                      _ptr(truncated), self._p_out[3], self._stream()))
 
+    def alloc_rollout_outputs(self, n_steps: int, traj: bool = False, terminal_kin: bool = False) -> dict:
+        """Caller-owned per-step output buffers for ``rollout(..., out=...)``: reward / terminated / truncated (K, E), and
+        ``traj`` / ``terminal_kin`` when asked for.  Reused across rollouts, a graph-captured planner loop allocates nothing."""
+        K, E, N = int(n_steps), self.E, self.N
+        kw = dict(device=self.device)
+        out = {"reward": torch.zeros((K, E), dtype=self.real, **kw),
+               "terminated": torch.zeros((K, E), dtype=torch.uint8, **kw),
+               "truncated": torch.zeros((K, E), dtype=torch.uint8, **kw)}
+        if traj:
+            out["traj"] = (torch.zeros((K, E, N, 20), dtype=self.real, **kw) if self.is_ctrl
+                           else torch.zeros((K, E, N, 12), dtype=torch.float32, **kw))
+        if terminal_kin:
+            out["terminal_kin"] = torch.zeros((K, E, N, 12), dtype=torch.float32, **kw)
+        return out
+
+    def rollout(self, actions: torch.Tensor, traj: bool = False, terminal_kin: bool = False, out: dict | None = None):
+        """``gpd_rollout``: K = ``actions.shape[0]`` control steps of the schedule ``actions`` (K, E, N, A) in one launch, the
+        same as K ``step`` calls whose intermediate observations are not read.  The final observation lands in the internal
+        ping-pong, as with ``step``.  Returns ``(obs, rewards (K,E), terminated (K,E), truncated (K,E))``, then ``traj``
+        ((K,E,N,12) kin rows, (K,E,N,20) for the Ctrl env) and ``terminal_kin`` ((K,E,N,12), written only where an env
+        finished; auto-reset RL envs) when asked for.  ``out``: buffers from ``alloc_rollout_outputs``, written in place."""
+        if actions.dtype != self.act_dtype or not actions.is_cuda or not actions.is_contiguous():
+            actions = actions.to(device=self.device, dtype=self.act_dtype).contiguous()
+        per_step = self.E * self.N * self.A
+        if actions.numel() == 0 or actions.numel() % per_step != 0:
+            raise ValueError(f"actions must have shape (K, {self.E}, {self.N}, {self.A}), got {tuple(actions.shape)}")
+        K = actions.numel() // per_step
+        if out is None:
+            out = self.alloc_rollout_outputs(K, traj, terminal_kin)
+        for name in ("reward", "terminated", "truncated") + (("traj",) if traj else ()) + (("terminal_kin",) if terminal_kin else ()):
+            t = out[name]
+            if t.shape[0] != K or not t.is_cuda or not t.is_contiguous():
+                raise ValueError(f"out[{name!r}] must be a contiguous CUDA tensor with K = {K} rows")
+        tr = out["traj"] if traj else None
+        tk = out["terminal_kin"] if terminal_kin else None
+        nxt = self._cur ^ 1
+        _lib.check(self.lib.gpd_rollout(self.h, int(K), _ptr(actions), self._p_obs[self._cur] if self._have_prev else None,
+                                        self._p_obs[nxt], _ptr(out["reward"]), _ptr(out["terminated"]),
+                                        _ptr(out["truncated"]), _ptr(tr), _ptr(tk), self._stream()))
+        self._cur, self._have_prev = nxt, True
+        res = (self.obs_buf[nxt], out["reward"], out["terminated"], out["truncated"])
+        if traj:
+            res += (tr,)
+        if terminal_kin:
+            res += (tk,)
+        return res
+
     def adopt_obs(self, obs: torch.Tensor):
         """Makes ``obs`` (the latest observation written by ``step_into``) the current internal observation."""
         self.obs_buf[self._cur].copy_(obs.reshape(self.obs_buf[self._cur].shape))

@@ -276,6 +276,26 @@ int gpd_force_downwash(int device, int precision, const gpd_drone_params* d, int
 int gpd_rollout_pid(gpd_sim* sim, int32_t n_ctrl_steps, const void* waypoints, int32_t n_wp,
                     int32_t* wp_counters, void* action, void* stream);
 
+/* K = n_steps control steps of BaseAviary.step with a given action schedule, in one launch.  Equivalent to
+ * K calls of gpd_step with actions[k], each reading the previous one's observation. The differences:
+ * only the final observation is written, and the per-step outputs land in rows of [K]-major arrays.
+ *   actions      dev [K][E][N][A], dtype as gpd_step; 16-byte aligned
+ *   obs_prev     as gpd_step (ring source of step 0; NULL = all-zero ring; ignored for the Ctrl env)
+ *   obs_out      dev [E][N][W]: the observation after step K-1; must not alias obs_prev; 16-byte aligned
+ *   reward       dev [K][E] Real or NULL;  terminated / truncated dev [K][E] uint8 or NULL
+ *   traj         dev or NULL: the device-computed part of each step's observation, i.e. what gpd_step would
+ *                have written there:
+ *                [K][E][N][12] float32 (RL envs: kin) or [K][E][N][20] Real (Ctrl env: the whole row)
+ *   terminal_kin dev [K][E][N][12] float32 or NULL: gpd_step's terminal_kin, per step (auto_reset, RL envs); rows of
+ *                steps where the env did not finish are left untouched
+ * Every configuration gpd_create accepts is supported. Auto-reset, episode statistics, counters and DSLPID
+ * state advance exactly as over K steps. The rollout is never launched programmatically behind a chained step, nor a
+ * step behind it; it allocates nothing and does not synchronise (graph-capturable). obs_out becomes the latest observation
+ * (gpd_get_state, the next gpd_step's obs_prev, a host mirror's rebuild). GPD_ERR_INVALID for n_steps < 1, a NULL
+ * actions / obs_out, aliased buffers, or actions / observations / traj / terminal_kin that are not 16-byte aligned. */
+int gpd_rollout(gpd_sim* sim, int32_t n_steps, const void* actions, const void* obs_prev, void* obs_out,
+                void* reward, uint8_t* terminated, uint8_t* truncated, void* traj, void* terminal_kin, void* stream);
+
 /* Diagnostics: number of CTAs of a step launch, and an optional device buffer [grid][8] of uint64 that every step
  * launch fills with per-CTA phase timestamps in ns (%globaltimer): 0 CTA start, 1 previous kernel complete (PDL wait
  * passed), 2 state+action arrived, 3 substeps done, 4 physics outputs stored, 5 history tile landed in shared memory
