@@ -67,7 +67,6 @@ static int fail(int code, const char* fmt, ...)
 // pinned host memory, log[row][col]: row = observation feature, col = drone.  The window of step t is rows [row, row + W):
 // 12 kin rows then the A*B ring rows, oldest -> newest.  A step slides the window by A rows: the device sends only what it
 // computed (12 kin rows, reward, flags); the newest action is written by the host from its own copy; nothing is echoed.
-enum { GPD_MIRROR_MAX_CHUNKS = 8 };
 struct Mirror {
     float* log = nullptr;
     int64_t rows = 0, ld = 0, col0 = 0;
@@ -79,10 +78,6 @@ struct Mirror {
     float* d_log = nullptr;         // device alias of the pinned log (cudaHostGetDevicePointer), or nullptr
     int zero_copy = 1;              // the step kernel reads the actions from and writes kin / reward / flags to pinned host memory itself
     float* d_full_t = nullptr;      // device [W][D], refresh scratch (lazy)
-    int chunks = 1;                 // a step is issued as `chunks` launches over CTA sub-ranges, each with its own copies
-    cudaStream_t cs[GPD_MIRROR_MAX_CHUNKS] = {};   // one stream per chunk: chunk c's H2D overlaps chunk c-1's kernel and D2H
-    cudaEvent_t ce[GPD_MIRROR_MAX_CHUNKS] = {};
-    cudaEvent_t ev_fork = nullptr;
     bool pending = false;           // a begin without its end
     const void* pending_obs = nullptr;
     const float* pending_actions = nullptr;
@@ -700,11 +695,6 @@ void gpd_destroy(gpd_sim* s)
     cudaFree(s->h_tkin); cudaFree(s->h_mask); cudaFree(s->stats_out); cudaFree(s->stats_gather);
     cudaFree(s->init_bufs[0]); cudaFree(s->init_bufs[1]); cudaFree(s->target_buf);
     cudaFree(s->mir.d_kin_t); cudaFree(s->mir.d_full_t);
-    for (int c = 0; c < GPD_MIRROR_MAX_CHUNKS; ++c) {
-        if (s->mir.cs[c]) cudaStreamDestroy(s->mir.cs[c]);
-        if (s->mir.ce[c]) cudaEventDestroy(s->mir.ce[c]);
-    }
-    if (s->mir.ev_fork) cudaEventDestroy(s->mir.ev_fork);
     delete s;
 }
 
@@ -766,8 +756,8 @@ static bool step_needs_sync(const gpd_sim* s, const void* actions, const void* o
 }
 
 static int step_impl(gpd_sim* s, const void* actions, const void* obs_prev, void* obs_out, void* reward, uint8_t* terminated,
-                     uint8_t* truncated, void* terminal_kin, float* kin_t, void* stream, int64_t cta0 = 0, int64_t ncta = 0,
-                     int64_t kin_ld = 0, bool host_io = false)
+                     uint8_t* truncated, void* terminal_kin, float* kin_t, void* stream, int64_t kin_ld = 0,
+                     bool host_io = false)
 {
     if (!s) return fail(GPD_ERR_INVALID, "null handle");
     if (!actions || !obs_out) return fail(GPD_ERR_INVALID, "gpd_step: actions and obs_out are required");
@@ -790,15 +780,13 @@ static int step_impl(gpd_sim* s, const void* actions, const void* obs_prev, void
     // (the two kernels agree bit for bit in FP64; in FP32 only up to the compiler's FMA contraction choices).
     const uintptr_t al_out = (uintptr_t)reward | (uintptr_t)terminated | (uintptr_t)truncated;
     const bool bulk = bulk_step(s, actions, obs_prev, obs_out);
-    // a step issued in chunks on several streams (ncta > 0) is synced by its caller, before the fork to the chunk streams
-    if (ncta == 0 && step_needs_sync(s, actions, obs_prev, obs_out)) {
+    if (step_needs_sync(s, actions, obs_prev, obs_out)) {
         int rc = sync_state(s, stream);
         if (rc) return rc;
         unchain(s, stream);
     }
     const int out_plain = ((al_out & 15) != 0 || host_io) ? 1 : 0;     // outputs in mapped host memory: plain stores by the threads
     LaunchCfg lc = bulk ? s->lc_bulk : s->lc;
-    if (ncta > 0) lc.grid = ncta;       // a sub-range of the CTAs (chunked host-mirror step); cta0 shifts the block index
     const void* prev_sim = nullptr;     // handle of the step kernel this one is chained behind
     if (s->tile_dep) {
         // programmatic launch only when the caller opted in (gpd_set_step_chaining) and the library's previous launch on this
@@ -813,32 +801,29 @@ static int step_impl(gpd_sim* s, const void* actions, const void* obs_prev, void
     // finer grain overlaps better (7.1 vs 8.5 us).  The per-tile words make the two mappings interchangeable.
     const int64_t tiles = lc.grid;
     int tpc = 1;
-    if (bulk && s->tile_dep && lc.pdl && ncta == 0 && s->bulk_tpc > 1 && prev_sim != (const void*)s) {
+    if (bulk && s->tile_dep && lc.pdl && s->bulk_tpc > 1 && prev_sim != (const void*)s) {
         tpc = s->bulk_tpc;
         lc.grid = (tiles + tpc - 1) / tpc;
     }
-    const bool last_chunk = cta0 + tiles >= s->lc.grid;
     if (s->cfg.precision == GPD_F64) {
         StepArgs<double> a = s->a64;
         a.actions = actions; a.obs_prev = (const float*)obs_prev; a.obs_out = obs_out; a.reward = (double*)reward;
         a.terminated = terminated; a.truncated = truncated; a.terminal_kin = (float*)terminal_kin; a.use_tma = use_tma;
-        a.kin_t = kin_t; a.kin_ld = kin_ld > 0 ? kin_ld : s->D; a.cta0 = (int32_t)cta0; a.out_plain = out_plain;
-        a.tpc = tpc; a.tile_end = (int32_t)(cta0 + tiles);
+        a.kin_t = kin_t; a.kin_ld = kin_ld > 0 ? kin_ld : s->D; a.out_plain = out_plain;
+        a.tpc = tpc; a.tile_end = (int32_t)tiles;
         if (bulk) CU(launch_step_bulk<double>(a, lc, st));
         else CU(launch_step<double>(a, lc, have ? &tp : nullptr, have ? &to : nullptr, have && s->tma_edge ? &te : nullptr, st));
     } else {
         StepArgs<float> a = s->a32;
         a.actions = actions; a.obs_prev = (const float*)obs_prev; a.obs_out = obs_out; a.reward = (float*)reward;
         a.terminated = terminated; a.truncated = truncated; a.terminal_kin = (float*)terminal_kin; a.use_tma = use_tma;
-        a.kin_t = kin_t; a.kin_ld = kin_ld > 0 ? kin_ld : s->D; a.cta0 = (int32_t)cta0; a.out_plain = out_plain;
-        a.tpc = tpc; a.tile_end = (int32_t)(cta0 + tiles);
+        a.kin_t = kin_t; a.kin_ld = kin_ld > 0 ? kin_ld : s->D; a.out_plain = out_plain;
+        a.tpc = tpc; a.tile_end = (int32_t)tiles;
         if (bulk) CU(launch_step_bulk<float>(a, lc, st));
         else CU(launch_step<float>(a, lc, have ? &tp : nullptr, have ? &to : nullptr, have && s->tma_edge ? &te : nullptr, st));
     }
-    if (last_chunk) {                     // the launch that covers the last CTA completes the step
-        s->last_obs = obs_out;
-        ++s->obs_seq;
-    }
+    s->last_obs = obs_out;
+    ++s->obs_seq;
     g_chain.set(s->cfg.device, st, true, capture_id(st), s);
     return GPD_OK;
 }
@@ -995,23 +980,6 @@ int gpd_mirror_attach(gpd_sim* s, float* log, int64_t rows, int64_t row_len, int
         if (!m.d_log) cudaGetLastError();
         if (const char* ev = getenv("GPD_MIRROR_ZEROCOPY")) m.zero_copy = atoi(ev) != 0;
     }
-    // Chunked issue (GPD_MIRROR_CHUNKS > 1): the step is cut into CTA sub-ranges on their own streams, so the action upload of
-    // chunk c+1 can overlap the kernel of chunk c and the result download of chunk c-1 (PCIe is full duplex).  Measured through
-    // the Python call site at 65,536 envs (profiles/r02): 139 / 147 / 166 / 193 us per step with 1 / 2 / 4 / 8 chunks — every
-    // chunk costs four more driver calls on the one host thread, which outweighs the overlap.  Default: one chunk.
-    int chunks = 1;
-    if (const char* ev = getenv("GPD_MIRROR_CHUNKS")) chunks = atoi(ev);
-    if (chunks > GPD_MIRROR_MAX_CHUNKS) chunks = GPD_MIRROR_MAX_CHUNKS;
-    if (chunks > s->lc.grid) chunks = (int)s->lc.grid;
-    if (chunks < 1) chunks = 1;
-    if (chunks > 1) {
-        for (int c = 0; c < chunks; ++c) {
-            if (!m.cs[c]) CU(cudaStreamCreateWithFlags(&m.cs[c], cudaStreamNonBlocking));
-            if (!m.ce[c]) CU(cudaEventCreateWithFlags(&m.ce[c], cudaEventDisableTiming));
-        }
-        if (!m.ev_fork) CU(cudaEventCreateWithFlags(&m.ev_fork, cudaEventDisableTiming));
-    }
-    m.chunks = chunks;
     return GPD_OK;
 }
 
@@ -1123,7 +1091,7 @@ int gpd_step_mirror_begin(gpd_sim* s, const void* actions, const void* d_obs_pre
     // One kernel launch per step instead of launch + three DMA operations, each with its own start-up latency, and the
     // transfers run under the kernel instead of behind it.  Anything not pinned falls back to staging + copies, per array.
     bool host_done = false;
-    if (m.chunks <= 1 && m.zero_copy && m.d_log) {
+    if (m.zero_copy && m.d_log) {
         // [reward | terminated | truncated] in one block (the facade's layout): one look-up covers all three
         const bool one_block = reward && (void*)terminated == (char*)reward + z.E * z.rs && truncated == terminated + z.E;
         void* a_rew = host_alias(reward);
@@ -1142,45 +1110,17 @@ int gpd_step_mirror_begin(gpd_sim* s, const void* actions, const void* d_obs_pre
             // kernel 105 us (the link delivers ~42 GB/s device-to-host on this pool: 3.5 MB = 84 us is the floor)
             float* kin_rows = m.d_log + (m.row + s->A) * m.ld + m.col0;
             int rc = step_impl(s, a_act, d_obs_prev, d_obs_out, a_rew, (uint8_t*)a_term, (uint8_t*)a_trunc, a_tkin, kin_rows, stream,
-                               0, 0, m.ld, true);
+                               m.ld, true);
             if (rc) return rc;
             host_done = true;
         }
     }
-    if (host_done) {
-        // nothing to copy
-    } else if (m.chunks <= 1) {
+    if (!host_done) {
         CU(cudaMemcpyAsync(s->h_act, actions, z.act_b, cudaMemcpyHostToDevice, st));
         int rc = step_impl(s, s->h_act, d_obs_prev, d_obs_out, d_rew, d_term, d_trunc, terminal_kin ? s->h_tkin : nullptr, m.d_kin_t, stream);
         if (rc) return rc;
         // what the device computed: 12 kin rows into the slid window
         CU(mirror_rows_d2h(s, m.row + s->A, m.d_kin_t, 12, st));
-    } else {
-        // fork: every chunk stream starts behind what the caller's stream holds so far (a window rebuild, earlier steps)
-        if (step_needs_sync(s, s->h_act, d_obs_prev, d_obs_out)) {      // ahead of the fork: every chunk stream waits for it
-            int rc = sync_state(s, stream);
-            if (rc) return rc;
-            unchain(s, stream);
-        }
-        CU(cudaEventRecord(m.ev_fork, st));
-        const int64_t G = s->lc.grid;
-        const size_t act_row = (size_t)s->A * 4;        // RL envs: float32 actions
-        for (int c = 0; c < m.chunks; ++c) {
-            const int64_t c0 = G * c / m.chunks, c1 = G * (c + 1) / m.chunks;
-            const int64_t d0 = c0 * s->dpb, d1 = c1 * s->dpb < s->D ? c1 * s->dpb : s->D;
-            cudaStream_t q = m.cs[c];
-            CU(cudaStreamWaitEvent(q, m.ev_fork, 0));
-            CU(cudaMemcpyAsync((char*)s->h_act + d0 * act_row, (const char*)actions + d0 * act_row, (size_t)(d1 - d0) * act_row,
-                               cudaMemcpyHostToDevice, q));
-            int rc = step_impl(s, s->h_act, d_obs_prev, d_obs_out, d_rew, d_term, d_trunc, terminal_kin ? s->h_tkin : nullptr,
-                               m.d_kin_t, (void*)q, c0, c1 - c0);
-            if (rc) return rc;
-            // this chunk's columns of the 12 kin rows
-            CU(cudaMemcpy2DAsync(m.log + (m.row + s->A) * m.ld + m.col0 + d0, (size_t)m.ld * sizeof(float), m.d_kin_t + d0,
-                                 (size_t)s->D * sizeof(float), (size_t)(d1 - d0) * sizeof(float), 12, cudaMemcpyDeviceToHost, q));
-            CU(cudaEventRecord(m.ce[c], q));
-        }
-        for (int c = 0; c < m.chunks; ++c) CU(cudaStreamWaitEvent(st, m.ce[c], 0));      // join
     }
     if (internal) { s->h_cur = nxt; s->h_has_prev = true; }
     // reward and flags of every env (one packed copy when the caller's arrays are laid out like the staging)

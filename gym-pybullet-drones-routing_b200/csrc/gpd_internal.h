@@ -113,7 +113,7 @@ struct StepArgs {
     unsigned long long* tile_seq;   // per-CTA step sequencing, one 64-bit word per tile at a 32-byte stride (tile_claim_and_wait)
     int32_t tile_dep;       // 1: a CTA waits only for ITS OWN tile's previous step (per-CTA flag) instead of the whole grid
     int32_t target_per_env; // 1: p.target holds D entries (per-env MultiHover targets), else N
-    int32_t cta0;           // first CTA of this launch (0 unless the step is issued in chunks)
+    int32_t cta0;           // block-index offset of a step launch: always 0 (dropping it from gpd::step_kernel measured 1 % slower on C4)
     int32_t out_plain;      // bulk path, per call: reward / terminated / truncated are not all 16-byte aligned -> plain stores by the threads
     int32_t tpc;            // bulk path, per call: tiles per CTA (0/1 = one; chained launches may take GPD_BULK_MAX_TPC)
     int32_t tile_end;       // bulk path, per call: first tile not covered by this launch

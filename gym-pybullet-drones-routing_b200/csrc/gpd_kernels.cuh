@@ -442,7 +442,7 @@ step_kernel(const __grid_constant__ StepArgs<R> a, const __grid_constant__ CUten
     const bool ctrl = a.env_kind == GPD_ENV_CTRL;
     Smem<R> sm{ smem_raw + a.tma_bytes, a.DPB, a.EPB, ctrl, MULTI };
     const int t = threadIdx.x;
-    const int bid = (int)blockIdx.x + a.cta0;     // a launch may cover a sub-range of the CTAs (chunked host-mirror steps)
+    const int bid = (int)blockIdx.x + a.cta0;     // a.cta0 is 0 (StepArgs)
     const int64_t row0 = (int64_t)bid * a.DPB;
     const int64_t d = row0 + t;
     const bool active = t < a.DPB && d < a.D;

@@ -34,22 +34,21 @@ def _kw(env_kind="hover", act="rpm", N=1, freq=30, flags=0, model=DroneModel.CF2
                 init_xyz=None, init_rpy=None)
 
 
-@pytest.mark.parametrize("act,N,freq,precision,chunks,io", [
-    ("rpm", 1, 30, "f32", 1, "zc"), ("rpm", 1, 30, "f32", 3, "zc"), ("rpm", 1, 48, "f64", 1, "zc"), ("pid", 1, 48, "f32", 4, "zc"),
-    ("one_d_rpm", 1, 30, "f32", 1, "zc"), ("rpm", 3, 30, "f32", 2, "zc"), ("vel", 2, 30, "f64", 1, "zc"),
-    ("rpm", 1, 30, "f32", 1, "zc_pinned_actions"), ("pid", 1, 48, "f64", 1, "zc_pinned_actions"), ("rpm", 2, 30, "f32", 1, "zc_pinned_actions"),
-    ("rpm", 1, 30, "f32", 1, "dma"), ("vel", 2, 30, "f64", 1, "dma"), ("rpm", 1, 30, "f32", 1, "pageable_outputs")])
-def test_cuda_host_mirror_equals_device_observation(act, N, freq, precision, chunks, io, monkeypatch):
+@pytest.mark.parametrize("act,N,freq,precision,io", [
+    ("rpm", 1, 30, "f32", "zc"), ("rpm", 1, 48, "f64", "zc"), ("pid", 1, 48, "f32", "zc"),
+    ("one_d_rpm", 1, 30, "f32", "zc"), ("rpm", 3, 30, "f32", "zc"), ("vel", 2, 30, "f64", "zc"),
+    ("rpm", 1, 30, "f32", "zc_pinned_actions"), ("pid", 1, 48, "f64", "zc_pinned_actions"), ("rpm", 2, 30, "f32", "zc_pinned_actions"),
+    ("rpm", 1, 30, "f32", "dma"), ("vel", 2, 30, "f64", "dma"), ("rpm", 1, 48, "f32", "dma"),
+    ("rpm", 1, 30, "f32", "pageable_outputs")])
+def test_cuda_host_mirror_equals_device_observation(act, N, freq, precision, io, monkeypatch):
     """The numpy-facing step returns a strided view of the pinned feature-major log; at every step it must equal, bit for bit,
     the device observation (same chain), through window slides, compactions (16-step log), masked and full resets, and
-    tensor-path steps in between (stale mirror -> rebuilt); also when the step is issued in chunks over CTA sub-ranges
-    (each with its own copies on its own stream).  io: "zc" = the zero-copy step (one chunk, pinned result arrays: the kernel
+    tensor-path steps in between (stale mirror -> rebuilt).  io: "zc" = the zero-copy step (pinned result arrays: the kernel
     writes kin rows / reward / flags / terminal rows straight into host memory; pageable actions are staged),
     "zc_pinned_actions" = it also reads the actions from host memory, "dma" = GPD_MIRROR_ZEROCOPY=0 (staging + copies),
     "pageable_outputs" = result arrays the device cannot address (falls back to staging + copies by itself)."""
     rng = np.random.default_rng(3)
     E = 517
-    monkeypatch.setenv("GPD_MIRROR_CHUNKS", str(chunks))
     if io == "dma":
         monkeypatch.setenv("GPD_MIRROR_ZEROCOPY", "0")
     kw = _kw("hover" if N == 1 else "multihover", act, N, freq, model=DroneModel.CF2P if act in ("pid", "vel") else DroneModel.CF2X)

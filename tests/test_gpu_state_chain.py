@@ -238,18 +238,15 @@ def test_state_chain_observation_is_state(monkeypatch):
     assert not torch.any(got[False][:, 0, 11] == 1.5)
 
 
-def test_state_chain_chunked_mirror(monkeypatch):
-    """Host-mirror steps issued in chunks on several streams (GPD_MIRROR_CHUNKS): chained steps, then a step whose obs_prev
-    is not the latest observation (a step_into that was not adopted), which must sync the state before the chunk streams
-    fork."""
+def test_state_chain_mirror_step_behind_a_foreign_obs_prev(monkeypatch):
+    """Host-mirror steps: chained steps, then a step whose obs_prev is not the latest observation (a step_into that was not
+    adopted), which must sync the state before it runs."""
     kw = se.shape("hover30")
     E = 5003
     P = Pairs(kw, E, 1, monkeypatch)
-    monkeypatch.setenv("GPD_MIRROR_CHUNKS", "2")
     for side in P.sides():
         side[0].reset()
         side[0].attach_mirror()
-    monkeypatch.delenv("GPD_MIRROR_CHUNKS")
     rng = np.random.default_rng(77)
     hacts = [rng.uniform(-1, 1, (E, 1, 4)).astype(np.float32) for _ in range(6)]
     dacts = rand_act(rng, E, 4)
@@ -262,7 +259,7 @@ def test_state_chain_chunked_mirror(monkeypatch):
     outs = [], []
     for j, side in enumerate(P.sides()):
         host_steps(side[0], hacts[:4], outs[j])
-    P.compare("chunked mirror steps", outs)
+    P.compare("mirror steps", outs)
     outs = [], []
     for j, side in enumerate(P.sides()):
         s = side[0]
@@ -272,5 +269,5 @@ def test_state_chain_chunked_mirror(monkeypatch):
         s.step_into(dacts, s.obs, out, rew, fl[0], fl[1])     # not adopted: the next mirror step reads another obs_prev
         host_steps(s, hacts[4:], outs[j])
         outs[j].extend([out, rew, fl])
-    P.check("chunked mirror step behind a foreign obs_prev", outs)
+    P.check("mirror step behind a foreign obs_prev", outs)
     P.close()
