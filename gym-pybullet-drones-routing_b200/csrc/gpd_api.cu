@@ -443,6 +443,27 @@ static int build_args(gpd_sim* s, StepArgs<R>& a)
     return upload_init(s, a, xyz.data(), rpy.data(), 0);
 }
 
+// gpd_plan: the copies of every env as PlanArgs, the handle's own StepArgs for everything else
+template <typename R>
+static cudaError_t plan_launch(const gpd_sim* s, const StepArgs<R>& src, int n_steps, int n_samples, const void* actions,
+                               const void* targets, double gamma, void* returns, int32_t* done_step, void* reward,
+                               void* final_kin, const LaunchCfg& lc, cudaStream_t st)
+{
+    StepArgs<R> a = src;
+    a.actions = actions;
+    PlanArgs<R> q{};
+    q.E = s->cfg.num_envs * (int64_t)n_samples;
+    q.D = q.E * s->cfg.num_drones;
+    q.n_samples = n_samples;
+    q.gamma = (R)gamma;
+    q.targets = (const R*)targets;
+    q.returns = (R*)returns;
+    q.done_step = done_step;
+    q.reward = (R*)reward;
+    q.final_kin = (float*)final_kin;
+    return launch_plan<R>(a, q, n_steps, lc, st);
+}
+
 extern "C" {
 
 int gpd_version(void) { return GPD_VERSION; }
@@ -1364,6 +1385,44 @@ int gpd_rollout(gpd_sim* s, int32_t n_steps, const void* actions, const void* ob
     }
     s->last_obs = obs_out;
     ++s->obs_seq;
+    return GPD_OK;
+}
+
+int gpd_plan(gpd_sim* s, int32_t n_steps, int32_t n_samples, const void* actions, const void* targets, double gamma,
+             void* returns, int32_t* done_step, void* reward, void* final_kin, void* stream)
+{
+    if (!s) return fail(GPD_ERR_INVALID, "null handle");
+    if (s->cfg.env_kind == GPD_ENV_CTRL) return fail(GPD_ERR_INVALID, "gpd_plan: the Ctrl env has no reward to plan on");
+    if (n_steps < 1 || n_samples < 1) return fail(GPD_ERR_INVALID, "gpd_plan: n_steps and n_samples must be >= 1");
+    if (!std::isfinite(gamma) || gamma < 0.0 || gamma > 1.0) return fail(GPD_ERR_INVALID, "gpd_plan: gamma must be in [0, 1]");
+    if (!actions || !returns) return fail(GPD_ERR_INVALID, "gpd_plan: actions and returns are required");
+    if (((uintptr_t)actions | (uintptr_t)final_kin) & 15)
+        return fail(GPD_ERR_INVALID, "gpd_plan: actions and final_kin must be 16-byte aligned");
+    const void* outs[4] = { returns, done_step, reward, final_kin };
+    for (int j = 0; j < 4; ++j) {
+        if (!outs[j]) continue;
+        if (outs[j] == actions || outs[j] == targets) return fail(GPD_ERR_INVALID, "gpd_plan: aliased buffers");
+        for (int k = j + 1; k < 4; ++k)
+            if (outs[j] == outs[k]) return fail(GPD_ERR_INVALID, "gpd_plan: aliased buffers");
+    }
+    // whole copies per CTA (MULTI) or DPB copies per CTA, as the rollout's tiles
+    const int N = s->cfg.num_drones;
+    const int64_t copies = s->cfg.num_envs * (int64_t)n_samples;
+    const int64_t per_cta = N > 1 ? s->dpb / N : s->dpb;
+    LaunchCfg lc{};
+    lc.threads = s->lc.threads - s->copy_threads;
+    lc.grid = (copies + per_cta - 1) / per_cta;
+    lc.smem = smem_bytes(s->cfg.precision == GPD_F64, false, N > 1, s->dpb, s->dpb / N);
+    if (lc.grid > INT32_MAX) return fail(GPD_ERR_INVALID, "gpd_plan: %lld copies need more than INT32_MAX CTAs", (long long)copies);
+    CU(use_device(s->cfg.device));
+    cudaStream_t st = (cudaStream_t)stream;
+    unchain(s, stream);                 // the next step is not launched programmatically behind the plan
+    int rc = sync_state(s, stream);     // chained-state tiles back into the arrays: the plan reads the state from there
+    if (rc) return rc;
+    if (s->cfg.precision == GPD_F64)
+        CU(plan_launch<double>(s, s->a64, n_steps, n_samples, actions, targets, gamma, returns, done_step, reward, final_kin, lc, st));
+    else
+        CU(plan_launch<float>(s, s->a32, n_steps, n_samples, actions, targets, gamma, returns, done_step, reward, final_kin, lc, st));
     return GPD_OK;
 }
 

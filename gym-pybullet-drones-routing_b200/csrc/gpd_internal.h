@@ -127,6 +127,20 @@ struct StepArgs {
     typename Vec4<R>::type* sR;   // [D] chained-state handles only: (rates.x, rates.y, rates.z, ep_ret)
 };
 
+// gpd_plan's own arguments, a separate kernel parameter so that StepArgs (every other kernel's parameter layout) is unchanged.
+// D / E count the copies: E = source envs * n_samples, D = E * N.  Outputs as in include/gpd.h.
+template <typename R>
+struct PlanArgs {
+    int64_t D, E;
+    int32_t n_samples;
+    R gamma;
+    const R* targets;       // [E_src][N][3] or nullptr (the handle's own)
+    R* returns;             // [E]
+    int32_t* done_step;     // [E] or nullptr
+    R* reward;              // [K][E] or nullptr
+    float* final_kin;       // [D][12] or nullptr
+};
+
 struct LaunchCfg {
     int threads;
     int64_t grid;
@@ -165,5 +179,8 @@ template <typename R> cudaError_t launch_rollout_pid(const StepArgs<R>& a, int n
                                                      int32_t* wp_counters, R* action, cudaStream_t st);
 // gpd_rollout: n_steps control steps of StepArgs::actions ([n_steps][D][A]) in one launch; traj as in include/gpd.h
 template <typename R> cudaError_t launch_rollout(const StepArgs<R>& a, int n_steps, void* traj, const LaunchCfg& lc, cudaStream_t st);
+// gpd_plan: n_steps control steps of q.n_samples copies of every env (StepArgs::actions [n_steps][E][S][N][A]), handle untouched
+template <typename R> cudaError_t launch_plan(const StepArgs<R>& a, const PlanArgs<R>& q, int n_steps, const LaunchCfg& lc,
+                                              cudaStream_t st);
 
 }  // namespace gpd

@@ -173,6 +173,14 @@ class BaseAviary:
             info = dict(info, traj=out[4])
         return obs, rew, term.view(torch.bool), trunc.view(torch.bool), info
 
+    def plan(self, actions, gamma: float = 1.0, targets=None, reward: bool = False, final_kin: bool = False,
+             out: dict | None = None) -> dict:
+        """Scores S candidate schedules per env from its current state without advancing the env (MPPI, CEM, random
+        shooting).  ``actions``: CUDA tensor (K, E, S, N, A).  Returns ``{"returns": (E, S), "done_step": (E, S)}``, plus
+        ``reward`` (K, E, S) and ``final_kin`` (E, S, N, 12) when asked for; see ``BatchedSim.plan``.  The env, its
+        observation and its episode statistics are left as they were."""
+        return self._sim.plan(actions, gamma=gamma, targets=targets, reward=reward, final_kin=final_kin, out=out)
+
     def render(self, mode='human', close=False):
         """Text output of env 0 (BaseAviary.py:387-412)."""
         st = self._state()[0][0].cpu().numpy()

@@ -240,6 +240,56 @@ class BatchedSim:
             res += (tk,)
         return res
 
+    def alloc_plan_outputs(self, n_steps: int, n_samples: int, reward: bool = False, final_kin: bool = False) -> dict:
+        """Caller-owned output buffers for ``plan(..., out=...)``: returns and done_step (E, S), and reward (K, E, S) /
+        final_kin (E, S, N, 12) when asked for.  Reused across plans, a graph-captured planner loop allocates nothing."""
+        K, S, E, N = int(n_steps), int(n_samples), self.E, self.N
+        kw = dict(device=self.device)
+        out = {"returns": torch.zeros((E, S), dtype=self.real, **kw),
+               "done_step": torch.zeros((E, S), dtype=torch.int32, **kw)}
+        if reward:
+            out["reward"] = torch.zeros((K, E, S), dtype=self.real, **kw)
+        if final_kin:
+            out["final_kin"] = torch.zeros((E, S, N, 12), dtype=torch.float32, **kw)
+        return out
+
+    def plan(self, actions: torch.Tensor, gamma: float = 1.0, targets: torch.Tensor | None = None, reward: bool = False,
+             final_kin: bool = False, out: dict | None = None) -> dict:
+        """``gpd_plan``: scores S candidate schedules per env from its current state, without advancing the env.
+        ``actions`` (K, E, S, N, A): sample s of env e runs K control steps of ``actions[:, e, s]`` on a copy of env e, with
+        no auto-reset.  Returns a dict with ``returns`` (E, S) (discounted by ``gamma``, up to and including the step that
+        ends the episode) and ``done_step`` (E, S) (that step, K if none), plus ``reward`` (K, E, S) and ``final_kin``
+        (E, S, N, 12) (the kin part of the last step's observation) when asked for.  ``targets`` (E, N, 3): target
+        positions for this plan only.  ``out``: buffers from ``alloc_plan_outputs``, written in place."""
+        if self.is_ctrl:
+            raise ValueError("the Ctrl env has no reward to plan on")
+        if actions.dim() != 5 or tuple(actions.shape[1:2] + actions.shape[3:]) != (self.E, self.N, self.A) or \
+                actions.shape[0] < 1 or actions.shape[2] < 1:
+            raise ValueError(f"actions must have shape (K, {self.E}, S, {self.N}, {self.A}), got {tuple(actions.shape)}")
+        K, S = int(actions.shape[0]), int(actions.shape[2])
+        if actions.dtype != self.act_dtype or not actions.is_cuda or not actions.is_contiguous():
+            actions = actions.to(device=self.device, dtype=self.act_dtype).contiguous()
+        if targets is not None and (tuple(targets.shape) != (self.E, self.N, 3) or targets.dtype != self.real or
+                                    not targets.is_contiguous()):
+            raise ValueError(f"targets must be a contiguous ({self.E}, {self.N}, 3) tensor of {self.real}")
+        if out is None:
+            out = self.alloc_plan_outputs(K, S, reward, final_kin)
+        want = {"returns": ((self.E, S), self.real), "done_step": ((self.E, S), torch.int32)}
+        if reward:
+            want["reward"] = ((K, self.E, S), self.real)
+        if final_kin:
+            want["final_kin"] = ((self.E, S, self.N, 12), torch.float32)
+        for name, (shape, dt) in want.items():
+            t = out.get(name)
+            if t is None or tuple(t.shape) != shape or t.dtype != dt or not t.is_contiguous():
+                raise ValueError(f"out[{name!r}] must be a contiguous {shape} tensor of {dt}")
+        if not all(t.is_cuda for t in [out[n] for n in want] + ([] if targets is None else [targets])):
+            raise ValueError("targets and the output buffers must be CUDA tensors")
+        _lib.check(self.lib.gpd_plan(self.h, K, S, _ptr(actions), _ptr(targets), float(gamma), _ptr(out["returns"]),
+                                     _ptr(out["done_step"]), _ptr(out.get("reward") if reward else None),
+                                     _ptr(out.get("final_kin") if final_kin else None), self._stream()))
+        return {name: out[name] for name in want}
+
     def adopt_obs(self, obs: torch.Tensor):
         """Makes ``obs`` (the latest observation written by ``step_into``) the current internal observation."""
         self.obs_buf[self._cur].copy_(obs.reshape(self.obs_buf[self._cur].shape))

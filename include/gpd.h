@@ -296,6 +296,31 @@ int gpd_rollout_pid(gpd_sim* sim, int32_t n_ctrl_steps, const void* waypoints, i
 int gpd_rollout(gpd_sim* sim, int32_t n_steps, const void* actions, const void* obs_prev, void* obs_out,
                 void* reward, uint8_t* terminated, uint8_t* truncated, void* traj, void* terminal_kin, void* stream);
 
+/* Planning rollouts (MPPI, CEM, random shooting): scores S = n_samples candidate schedules of K = n_steps control steps per
+ * env, from the env's current state, without advancing the env.  Sample s of env e is exactly a copy of env e that starts
+ * from the state the next gpd_step of env e would start from (pos, quat, vel, body rates, previous RPM for drag, DSLPID
+ * state, step counter, per-env target) and runs BaseAviary.step (BaseAviary.py:259-383) with actions[k][e][s] for
+ * k = 0..K-1, with NO auto-reset whatever the handle's auto_reset.  Reward and flags are HoverAviary.py:68-117 /
+ * MultiHoverAviary.py:84-130; truncation uses the copy's counter, advanced by the substeps per step as in gpd_step
+ * (HoverAviary.py:114).  The handle is not modified: state, counters, episode return and statistics, the latest
+ * observation, the aux copies and a host mirror stay as they were.  Real = the handle's precision.
+ *   actions   dev [K][E][S][N][A] float32 (the RL action dtype); 16-byte aligned
+ *   targets   dev [E][N][3] Real or NULL: overrides the handle's targets for this plan only (NULL = the handle's own,
+ *             shared or per env)
+ *   returns   dev [E][S] Real, required: G = 0, w = 1; for k = 0..K-1, while the copy has not ended: G = G + w * r_k, then
+ *             the copy ends if terminated_k | truncated_k, else w = w * (Real)gamma.  Each operation is rounded in Real, no
+ *             fused multiply-add.  The reward of the step that ends the episode is included.
+ *   done_step dev [E][S] int32 or NULL: the first k with terminated | truncated; K if none
+ *   reward    dev [K][E][S] Real or NULL: every step's reward, also after done_step (the copy keeps stepping)
+ *   final_kin dev [E][S][N][12] float32 or NULL: the kin part of the observation gpd_step would write at step K-1
+ *             (terminal-value bootstrap); 16-byte aligned
+ * The plan is never launched programmatically behind a chained step, nor a step behind it; it allocates nothing and does
+ * not synchronise (graph-capturable).  GPD_ERR_INVALID for the Ctrl env, n_steps < 1, n_samples < 1, gamma not finite or
+ * outside [0, 1], a NULL actions / returns, unaligned actions / final_kin, aliased output buffers, or more than INT32_MAX
+ * CTAs of copies. */
+int gpd_plan(gpd_sim* sim, int32_t n_steps, int32_t n_samples, const void* actions, const void* targets, double gamma,
+             void* returns, int32_t* done_step, void* reward, void* final_kin, void* stream);
+
 /* Diagnostics: number of CTAs of a step launch, and an optional device buffer [grid][8] of uint64 that every step
  * launch fills with per-CTA phase timestamps in ns (%globaltimer): 0 CTA start, 1 previous kernel complete (PDL wait
  * passed), 2 state+action arrived, 3 substeps done, 4 physics outputs stored, 5 history tile landed in shared memory
