@@ -31,7 +31,7 @@ SYMBOLS = [
     "gpd_set_timeline_buffer", "gpd_count_nonfinite", "gpd_set_targets", "gpd_mirror_alloc", "gpd_mirror_free",
     "gpd_mirror_attach", "gpd_mirror_row", "gpd_step_mirror", "gpd_step_mirror_begin", "gpd_step_mirror_end",
     "gpd_reset_mirror", "gpd_nccl_unique_id", "gpd_nccl_comm_init", "gpd_nccl_comm_destroy", "gpd_adjacency",
-    "gpd_set_step_chaining", "gpd_rollout", "gpd_plan",
+    "gpd_set_step_chaining", "gpd_rollout", "gpd_plan", "gpd_plan_grad_tape_bytes", "gpd_plan_grad",
 ]
 
 
@@ -156,6 +156,9 @@ def load(path: str | None = None):
     L.gpd_rollout_pid.argtypes = [vp, i32, vp, i32, vp, vp, vp]
     L.gpd_rollout.argtypes = [vp, i32, vp, vp, vp, vp, u8p, u8p, vp, vp, vp]
     L.gpd_plan.argtypes = [vp, i32, i32, vp, vp, dbl, vp, vp, vp, vp, vp]
+    L.gpd_plan_grad_tape_bytes.argtypes = [vp, i32, i32]
+    L.gpd_plan_grad_tape_bytes.restype = i64
+    L.gpd_plan_grad.argtypes = [vp, i32, i32, vp, vp, dbl, vp, vp, vp, vp, i64, vp]
     L.gpd_episode_stats.argtypes = [vp, C.POINTER(dbl), C.c_int, vp, vp]
     L.gpd_set_targets.argtypes = [vp, C.POINTER(dbl), C.c_int]
     L.gpd_mirror_alloc.argtypes = [i64, i64, C.POINTER(vp)]

@@ -464,6 +464,36 @@ static cudaError_t plan_launch(const gpd_sim* s, const StepArgs<R>& src, int n_s
     return launch_plan<R>(a, q, n_steps, lc, st);
 }
 
+// gpd_plan_grad: gpd_plan's copies with the gradient and the tape
+template <typename R>
+static cudaError_t plan_grad_launch(const gpd_sim* s, const StepArgs<R>& src, int n_steps, int n_samples, const void* actions,
+                                    const void* targets, double gamma, void* returns, int32_t* done_step, void* grad,
+                                    void* tape, const LaunchCfg& lc, cudaStream_t st)
+{
+    StepArgs<R> a = src;
+    a.actions = actions;
+    PlanGradArgs<R> q{};
+    q.E = s->cfg.num_envs * (int64_t)n_samples;
+    q.D = q.E * s->cfg.num_drones;
+    q.n_samples = n_samples;
+    q.gamma = (R)gamma;
+    q.targets = (const R*)targets;
+    q.returns = (R*)returns;
+    q.done_step = done_step;
+    q.grad = (R*)grad;
+    q.tape = (R*)tape;
+    return launch_plan_grad<R>(a, q, n_steps, lc, st);
+}
+
+// the tape of gpd_plan_grad: 13 Reals per copy drone and control step
+static int64_t plan_grad_tape_bytes(const gpd_sim* s, int32_t n_steps, int32_t n_samples)
+{
+    const int64_t D = s->cfg.num_envs * (int64_t)n_samples * s->cfg.num_drones;
+    const int64_t rs = s->cfg.precision == GPD_F64 ? 8 : 4;
+    if (D > INT64_MAX / 13 / rs / n_steps) return -1;
+    return (int64_t)n_steps * 13 * D * rs;
+}
+
 extern "C" {
 
 int gpd_version(void) { return GPD_VERSION; }
@@ -1423,6 +1453,58 @@ int gpd_plan(gpd_sim* s, int32_t n_steps, int32_t n_samples, const void* actions
         CU(plan_launch<double>(s, s->a64, n_steps, n_samples, actions, targets, gamma, returns, done_step, reward, final_kin, lc, st));
     else
         CU(plan_launch<float>(s, s->a32, n_steps, n_samples, actions, targets, gamma, returns, done_step, reward, final_kin, lc, st));
+    return GPD_OK;
+}
+
+int64_t gpd_plan_grad_tape_bytes(const gpd_sim* s, int32_t n_steps, int32_t n_samples)
+{
+    if (!s) return fail(GPD_ERR_INVALID, "null handle");
+    if (n_steps < 1 || n_samples < 1) return fail(GPD_ERR_INVALID, "gpd_plan_grad_tape_bytes: n_steps and n_samples must be >= 1");
+    const int64_t b = plan_grad_tape_bytes(s, n_steps, n_samples);
+    if (b < 0) return fail(GPD_ERR_INVALID, "gpd_plan_grad_tape_bytes: the tape does not fit in 63 bits");
+    return b;
+}
+
+int gpd_plan_grad(gpd_sim* s, int32_t n_steps, int32_t n_samples, const void* actions, const void* targets, double gamma,
+                  void* returns, int32_t* done_step, void* grad_actions, void* tape, int64_t tape_bytes, void* stream)
+{
+    if (!s) return fail(GPD_ERR_INVALID, "null handle");
+    const gpd_config& c = s->cfg;
+    if (c.env_kind == GPD_ENV_CTRL) return fail(GPD_ERR_INVALID, "gpd_plan_grad: the Ctrl env has no reward to plan on");
+    if (c.action_type != GPD_ACT_RPM && c.action_type != GPD_ACT_ONE_D_RPM)
+        return fail(GPD_ERR_INVALID, "gpd_plan_grad: only the RPM and ONE_D_RPM actions are differentiated (no DSLPID adjoint)");
+    if (c.physics_flags != 0)
+        return fail(GPD_ERR_INVALID, "gpd_plan_grad: only Physics.DYN (physics_flags 0) is differentiated, no force models");
+    if (n_steps < 1 || n_samples < 1) return fail(GPD_ERR_INVALID, "gpd_plan_grad: n_steps and n_samples must be >= 1");
+    if (!std::isfinite(gamma) || gamma < 0.0 || gamma > 1.0) return fail(GPD_ERR_INVALID, "gpd_plan_grad: gamma must be in [0, 1]");
+    if (!actions || !returns || !grad_actions || !tape)
+        return fail(GPD_ERR_INVALID, "gpd_plan_grad: actions, returns, grad_actions and tape are required");
+    if (((uintptr_t)actions | (uintptr_t)tape) & 15)
+        return fail(GPD_ERR_INVALID, "gpd_plan_grad: actions and tape must be 16-byte aligned");
+    const int64_t need = plan_grad_tape_bytes(s, n_steps, n_samples);
+    if (need < 0 || tape_bytes < need)
+        return fail(GPD_ERR_INVALID, "gpd_plan_grad: tape_bytes %lld < %lld", (long long)tape_bytes, (long long)need);
+    const void* bufs[6] = { actions, targets, returns, done_step, grad_actions, tape };
+    for (int j = 0; j < 6; ++j)
+        for (int k = j + 1; k < 6; ++k)
+            if (bufs[j] && bufs[j] == bufs[k]) return fail(GPD_ERR_INVALID, "gpd_plan_grad: aliased buffers");
+    const int N = c.num_drones;
+    const int64_t copies = c.num_envs * (int64_t)n_samples;
+    const int64_t per_cta = N > 1 ? s->dpb / N : s->dpb;
+    LaunchCfg lc{};
+    lc.threads = s->lc.threads - s->copy_threads;
+    lc.grid = (copies + per_cta - 1) / per_cta;
+    lc.smem = smem_bytes(c.precision == GPD_F64, false, N > 1, s->dpb, s->dpb / N);
+    if (lc.grid > INT32_MAX) return fail(GPD_ERR_INVALID, "gpd_plan_grad: %lld copies need more than INT32_MAX CTAs", (long long)copies);
+    CU(use_device(c.device));
+    cudaStream_t st = (cudaStream_t)stream;
+    unchain(s, stream);                 // the next step is not launched programmatically behind the plan
+    int rc = sync_state(s, stream);     // chained-state tiles back into the arrays: the plan reads the state from there
+    if (rc) return rc;
+    if (c.precision == GPD_F64)
+        CU(plan_grad_launch<double>(s, s->a64, n_steps, n_samples, actions, targets, gamma, returns, done_step, grad_actions, tape, lc, st));
+    else
+        CU(plan_grad_launch<float>(s, s->a32, n_steps, n_samples, actions, targets, gamma, returns, done_step, grad_actions, tape, lc, st));
     return GPD_OK;
 }
 

@@ -141,6 +141,19 @@ struct PlanArgs {
     float* final_kin;       // [D][12] or nullptr
 };
 
+// gpd_plan_grad's own arguments (PlanArgs' copy counts and return outputs, the gradient and the tape)
+template <typename R>
+struct PlanGradArgs {
+    int64_t D, E;
+    int32_t n_samples;
+    R gamma;
+    const R* targets;       // [E_src][N][3] or nullptr (the handle's own)
+    R* returns;             // [E]
+    int32_t* done_step;     // [E] or nullptr
+    R* grad;                // [K][D][A]
+    R* tape;                // [K][13][D]: each copy drone's state at the start of every control step
+};
+
 struct LaunchCfg {
     int threads;
     int64_t grid;
@@ -182,5 +195,8 @@ template <typename R> cudaError_t launch_rollout(const StepArgs<R>& a, int n_ste
 // gpd_plan: n_steps control steps of q.n_samples copies of every env (StepArgs::actions [n_steps][E][S][N][A]), handle untouched
 template <typename R> cudaError_t launch_plan(const StepArgs<R>& a, const PlanArgs<R>& q, int n_steps, const LaunchCfg& lc,
                                               cudaStream_t st);
+// gpd_plan_grad: gpd_plan's returns of a LEAN configuration and their gradient with respect to the actions (q.grad)
+template <typename R> cudaError_t launch_plan_grad(const StepArgs<R>& a, const PlanGradArgs<R>& q, int n_steps,
+                                                   const LaunchCfg& lc, cudaStream_t st);
 
 }  // namespace gpd

@@ -181,6 +181,12 @@ class BaseAviary:
         observation and its episode statistics are left as they were."""
         return self._sim.plan(actions, gamma=gamma, targets=targets, reward=reward, final_kin=final_kin, out=out)
 
+    def plan_grad(self, actions, gamma: float = 1.0, targets=None, out: dict | None = None) -> dict:
+        """``plan``'s returns and done_step together with ``grad`` (K, E, S, N, A), the gradient of each candidate's
+        return with respect to its actions (gradient-based shooting MPC), without advancing the env.  Physics.DYN with
+        RPM or ONE_D_RPM actions only; see ``BatchedSim.plan_grad`` and ``BatchedSim.plan_return``."""
+        return self._sim.plan_grad(actions, gamma=gamma, targets=targets, out=out)
+
     def render(self, mode='human', close=False):
         """Text output of env 0 (BaseAviary.py:387-412)."""
         st = self._state()[0][0].cpu().numpy()

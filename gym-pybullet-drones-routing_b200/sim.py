@@ -22,6 +22,48 @@ def _ptr(t):
     return None if t is None else C.c_void_p(t.data_ptr())
 
 
+def _plan_inputs(sim, actions, targets):
+    """The checks ``plan`` and ``plan_grad`` share: actions (K, E, S, N, A) in the action dtype on the device, targets."""
+    if sim.is_ctrl:
+        raise ValueError("the Ctrl env has no reward to plan on")
+    if actions.dim() != 5 or tuple(actions.shape[1:2] + actions.shape[3:]) != (sim.E, sim.N, sim.A) or \
+            actions.shape[0] < 1 or actions.shape[2] < 1:
+        raise ValueError(f"actions must have shape (K, {sim.E}, S, {sim.N}, {sim.A}), got {tuple(actions.shape)}")
+    K, S = int(actions.shape[0]), int(actions.shape[2])
+    if actions.dtype != sim.act_dtype or not actions.is_cuda or not actions.is_contiguous():
+        actions = actions.to(device=sim.device, dtype=sim.act_dtype).contiguous()
+    if targets is not None and (tuple(targets.shape) != (sim.E, sim.N, 3) or targets.dtype != sim.real or
+                                not targets.is_contiguous()):
+        raise ValueError(f"targets must be a contiguous ({sim.E}, {sim.N}, 3) tensor of {sim.real}")
+    return actions, K, S
+
+
+def _plan_outputs(out, want, targets):
+    """Output buffers of ``plan`` / ``plan_grad``: ``want`` maps each name to its (shape, dtype)."""
+    for name, (shape, dt) in want.items():
+        t = out.get(name)
+        if t is None or tuple(t.shape) != shape or t.dtype != dt or not t.is_contiguous():
+            raise ValueError(f"out[{name!r}] must be a contiguous {shape} tensor of {dt}")
+    if not all(t.is_cuda for t in [out[n] for n in want] + ([] if targets is None else [targets])):
+        raise ValueError("targets and the output buffers must be CUDA tensors")
+
+
+class _PlanReturn(torch.autograd.Function):
+    """``BatchedSim.plan_return``: forward ``gpd_plan_grad``'s returns, backward its gradient."""
+
+    @staticmethod
+    def forward(ctx, sim, actions, gamma, targets):
+        res = sim.plan_grad(actions.detach(), gamma=gamma, targets=targets)
+        ctx.save_for_backward(res["grad"])
+        ctx.act_dtype = actions.dtype
+        return res["returns"]
+
+    @staticmethod
+    def backward(ctx, grad_output):
+        (grad,) = ctx.saved_tensors
+        return None, (grad_output[None, :, :, None, None] * grad).to(ctx.act_dtype), None, None
+
+
 class HostMirror:
     """Feature-major observation log in pinned host memory (``gpd_mirror_alloc``; layout in ``include/gpd.h``).
 
@@ -66,6 +108,7 @@ class BatchedSim:
         self.device_index = int(device)
         self.device = torch.device("cuda", self.device_index)
         self.auto_reset = bool(auto_reset)
+        self.physics_flags = int(physics_flags)
         cfg = _lib.ConfigC()
         cfg.device = self.device_index
         cfg.precision = _lib.GPD_F64 if precision == "f64" else _lib.GPD_F32
@@ -261,17 +304,7 @@ class BatchedSim:
         ends the episode) and ``done_step`` (E, S) (that step, K if none), plus ``reward`` (K, E, S) and ``final_kin``
         (E, S, N, 12) (the kin part of the last step's observation) when asked for.  ``targets`` (E, N, 3): target
         positions for this plan only.  ``out``: buffers from ``alloc_plan_outputs``, written in place."""
-        if self.is_ctrl:
-            raise ValueError("the Ctrl env has no reward to plan on")
-        if actions.dim() != 5 or tuple(actions.shape[1:2] + actions.shape[3:]) != (self.E, self.N, self.A) or \
-                actions.shape[0] < 1 or actions.shape[2] < 1:
-            raise ValueError(f"actions must have shape (K, {self.E}, S, {self.N}, {self.A}), got {tuple(actions.shape)}")
-        K, S = int(actions.shape[0]), int(actions.shape[2])
-        if actions.dtype != self.act_dtype or not actions.is_cuda or not actions.is_contiguous():
-            actions = actions.to(device=self.device, dtype=self.act_dtype).contiguous()
-        if targets is not None and (tuple(targets.shape) != (self.E, self.N, 3) or targets.dtype != self.real or
-                                    not targets.is_contiguous()):
-            raise ValueError(f"targets must be a contiguous ({self.E}, {self.N}, 3) tensor of {self.real}")
+        actions, K, S = _plan_inputs(self, actions, targets)
         if out is None:
             out = self.alloc_plan_outputs(K, S, reward, final_kin)
         want = {"returns": ((self.E, S), self.real), "done_step": ((self.E, S), torch.int32)}
@@ -279,16 +312,58 @@ class BatchedSim:
             want["reward"] = ((K, self.E, S), self.real)
         if final_kin:
             want["final_kin"] = ((self.E, S, self.N, 12), torch.float32)
-        for name, (shape, dt) in want.items():
-            t = out.get(name)
-            if t is None or tuple(t.shape) != shape or t.dtype != dt or not t.is_contiguous():
-                raise ValueError(f"out[{name!r}] must be a contiguous {shape} tensor of {dt}")
-        if not all(t.is_cuda for t in [out[n] for n in want] + ([] if targets is None else [targets])):
-            raise ValueError("targets and the output buffers must be CUDA tensors")
+        _plan_outputs(out, want, targets)
         _lib.check(self.lib.gpd_plan(self.h, K, S, _ptr(actions), _ptr(targets), float(gamma), _ptr(out["returns"]),
                                      _ptr(out["done_step"]), _ptr(out.get("reward") if reward else None),
                                      _ptr(out.get("final_kin") if final_kin else None), self._stream()))
         return {name: out[name] for name in want}
+
+    def plan_grad_tape_bytes(self, n_steps: int, n_samples: int) -> int:
+        """Bytes of the workspace ``plan_grad`` needs for ``n_steps`` x ``n_samples`` copies of every env."""
+        b = self.lib.gpd_plan_grad_tape_bytes(self.h, int(n_steps), int(n_samples))
+        _lib.check(b if b < 0 else 0)
+        return int(b)
+
+    def alloc_plan_grad_outputs(self, n_steps: int, n_samples: int) -> dict:
+        """Caller-owned buffers for ``plan_grad(..., out=...)``: returns and done_step (E, S), grad (K, E, S, N, A) and the
+        tape (a uint8 workspace of ``plan_grad_tape_bytes`` bytes).  Reused across calls, a graph-captured planner
+        allocates nothing."""
+        K, S, E, N, A = int(n_steps), int(n_samples), self.E, self.N, self.A
+        kw = dict(device=self.device)
+        return {"returns": torch.zeros((E, S), dtype=self.real, **kw),
+                "done_step": torch.zeros((E, S), dtype=torch.int32, **kw),
+                "grad": torch.zeros((K, E, S, N, A), dtype=self.real, **kw),
+                "tape": torch.empty(self.plan_grad_tape_bytes(K, S), dtype=torch.uint8, **kw)}
+
+    def plan_grad(self, actions: torch.Tensor, gamma: float = 1.0, targets: torch.Tensor | None = None,
+                  out: dict | None = None) -> dict:
+        """``gpd_plan_grad``: ``plan``'s returns and done_step, and ``grad`` (K, E, S, N, A) in the handle's precision, the
+        gradient of each copy's return with respect to its actions (flags and end step held constant, rows after the
+        end step 0; include/gpd.h).  Physics.DYN with RPM or ONE_D_RPM actions on Hover / MultiHover only.  Arguments as
+        for ``plan``; ``out``: buffers from ``alloc_plan_grad_outputs``, written in place."""
+        if self.is_ctrl or self.action_type not in ("rpm", "one_d_rpm") or self.physics_flags != 0:
+            raise ValueError("plan_grad differentiates Physics.DYN (physics_flags 0) with rpm / one_d_rpm actions on the "
+                             "Hover and MultiHover envs only")
+        actions, K, S = _plan_inputs(self, actions, targets)
+        if out is None:
+            out = self.alloc_plan_grad_outputs(K, S)
+        want = {"returns": ((self.E, S), self.real), "done_step": ((self.E, S), torch.int32),
+                "grad": ((K, self.E, S, self.N, self.A), self.real)}
+        _plan_outputs(out, want, targets)
+        tape = out.get("tape")
+        need = self.plan_grad_tape_bytes(K, S)
+        if tape is None or tape.dim() != 1 or tape.dtype != torch.uint8 or tape.numel() < need or not tape.is_cuda:
+            raise ValueError(f"out['tape'] must be a CUDA uint8 tensor of at least {need} bytes")
+        _lib.check(self.lib.gpd_plan_grad(self.h, K, S, _ptr(actions), _ptr(targets), float(gamma), _ptr(out["returns"]),
+                                          _ptr(out["done_step"]), _ptr(out["grad"]), _ptr(tape), tape.numel(),
+                                          self._stream()))
+        return {name: out[name] for name in want}
+
+    def plan_return(self, actions: torch.Tensor, gamma: float = 1.0, targets: torch.Tensor | None = None) -> torch.Tensor:
+        """The (E, S) returns of ``plan_grad`` as a differentiable function of ``actions`` (K, E, S, N, A): its backward
+        is ``grad_output[None, :, :, None, None] * grad``, cast to the actions' dtype, so torch optimisers and losses use
+        the kernel's gradient directly."""
+        return _PlanReturn.apply(self, actions, float(gamma), targets)
 
     def adopt_obs(self, obs: torch.Tensor):
         """Makes ``obs`` (the latest observation written by ``step_into``) the current internal observation."""

@@ -321,6 +321,29 @@ int gpd_rollout(gpd_sim* sim, int32_t n_steps, const void* actions, const void* 
 int gpd_plan(gpd_sim* sim, int32_t n_steps, int32_t n_samples, const void* actions, const void* targets, double gamma,
              void* returns, int32_t* done_step, void* reward, void* final_kin, void* stream);
 
+/* Planning gradients (gradient-based shooting MPC, MPPI with a gradient refinement step): gpd_plan's returns and done_step
+ * together with the gradient of every copy's discounted return with respect to its action schedule, in one launch.
+ *   actions, targets, gamma, returns, done_step: as for gpd_plan.  In FP64 returns and done_step are bit-identical to
+ *             gpd_plan's for the same inputs; in FP32 they are within gpd_plan's FP32 ceilings.
+ *   grad_actions dev [K][E][S][N][A] Real, required: entry [k][e][s][i][j] = dG_{e,s} / d actions[k][e][s][i][j].
+ *   tape      dev workspace of at least gpd_plan_grad_tape_bytes(sim, K, S) bytes, 16-byte aligned, required; its layout
+ *             is private (each copy's state at the start of every control step).  The call allocates nothing.
+ * The derivative holds the end step and the terminated / truncated flags constant, so the gradient is
+ * sum_{k'=k..done_step} w_k' dr_k'/da_k (w_k' the return's weights), and every row with k > done_step is exactly 0.  The
+ * reward's clip r = v > 0 ? v : 0 contributes dv only where v > 0, as the kernel branches.  _integrateQ
+ * (BaseAviary.py:876-889) is differentiated as its smooth update cos(theta) I + (sin(theta)/|w|) Lambda(w), theta =
+ * |w| dt/2, extended to |w| -> 0 by its power series: the reference's early return for |w| <= 1e-8 is not differentiated
+ * (otherwise a drone at hover with equal rotor actions would report dq/dw = 0, which finite differences contradict).
+ * Supported: GPD_ENV_HOVER and GPD_ENV_MULTIHOVER, GPD_ACT_RPM and GPD_ACT_ONE_D_RPM, physics_flags == 0, FP32 and FP64,
+ * every drone model and pyb_freq / ctrl_freq.  GPD_ERR_INVALID for anything else (the Ctrl env, DSLPID-family actions,
+ * force models), and as gpd_plan for n_steps < 1, n_samples < 1, gamma not finite or outside [0, 1], a NULL actions /
+ * returns / grad_actions / tape, a tape_bytes too small, unaligned actions / tape, aliasing between any two of actions,
+ * targets and the outputs, or more than INT32_MAX CTAs of copies.  The handle is not modified; chained-state tiles are
+ * synced first and the stream is unchained; the call does not synchronise (graph-capturable). */
+int64_t gpd_plan_grad_tape_bytes(const gpd_sim* sim, int32_t n_steps, int32_t n_samples);
+int gpd_plan_grad(gpd_sim* sim, int32_t n_steps, int32_t n_samples, const void* actions, const void* targets, double gamma,
+                  void* returns, int32_t* done_step, void* grad_actions, void* tape, int64_t tape_bytes, void* stream);
+
 /* Diagnostics: number of CTAs of a step launch, and an optional device buffer [grid][8] of uint64 that every step
  * launch fills with per-CTA phase timestamps in ns (%globaltimer): 0 CTA start, 1 previous kernel complete (PDL wait
  * passed), 2 state+action arrived, 3 substeps done, 4 physics outputs stored, 5 history tile landed in shared memory

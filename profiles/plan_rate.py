@@ -34,6 +34,7 @@ SHAPES = {
     "C2": dict(env_kind="hover", action_type="rpm", N=1, pyb=240, ctrl=30, phy=0, precision="f32"),
     "C5": dict(env_kind="hover", action_type="pid", N=1, pyb=240, ctrl=48, phy=0, precision="f32"),
     "C3": dict(env_kind="multihover", action_type="rpm", N=2, pyb=240, ctrl=30, phy=3, precision="f64"),
+    "C3dyn": dict(env_kind="multihover", action_type="rpm", N=2, pyb=240, ctrl=30, phy=0, precision="f64"),   # plan_grad_rate.py
 }
 RUNS = [("C2", 1024, 256, 32), ("C2", 64, 4096, 16), ("C5", 1024, 256, 16), ("C3", 1024, 32, 32)]
 
